@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — entity-steps/s of the B200 six_dof() RK4 path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--worlds M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--worlds M] [--dump-outputs DIR]
 
 One "step" = one RK4 tick of the hot path over the whole batch of synthetic worlds
 (one body kernel launch, the state streaming HBM -> registers -> HBM).  Workload at
@@ -47,6 +47,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark only reads the tree build() left (it may be read-only)
 
 import numpy as np
 
@@ -177,7 +178,6 @@ def cpu_arm(steps: int, warmup: int, target_s: float):
     of two (2^12..2^22 = the GPU arm's batch) that keeps `steps` ticks near `target_s` seconds on this host."""
     from oracle import oracle as O
 
-    O.build()
     threads = min(O.max_threads(), effective_cores())
     r1, _ = cpu_oracle_run(1 << 12, 100, 1)                      # one thread, 0.2 s
     rN, _ = cpu_oracle_run(1 << 16, 40, threads)                 # calibration, all threads
@@ -331,21 +331,23 @@ def run_baseline_configs(args, torch, el, stream, local, rank, world_size):
     return out
 
 
-def ensure_built():
-    """Harness step: (re)build the in-tree CUDA library if its sources are newer (make is a no-op otherwise)."""
-    import fcntl
+DUMP_WORLDS = 1 << 16  # worlds sampled by --dump-outputs: 4 f64 columns x 2^16 worlds = 13 MB
 
-    try:
-        with open(os.path.join(ROOT, "elodin_b200", "csrc", ".build.lock"), "w") as lock:
-            fcntl.flock(lock, fcntl.LOCK_EX)  # ranks of one node take turns; all but the first find it up to date
-            subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "elodin_b200", "csrc")], check=True,
-                           stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    except Exception:
-        pass  # the import below fails loudly if the library is really missing
+
+def dump_outputs(ex, out_dir: str):
+    """Write the columns a caller of the timed executor downloads (WorldPos, WorldVel, WorldAccel, Force) as
+    <out_dir>/<column>.npy, float64 [worlds, 1, width], for a fixed, seeded sample of DUMP_WORLDS worlds in
+    ascending order (every world when the batch is smaller)."""
+    from elodin_b200.executor import FORCE, WORLD_ACCEL, WORLD_POS, WORLD_VEL
+
+    M = ex.n_worlds
+    idx = np.sort(np.random.default_rng(0).choice(M, size=min(M, DUMP_WORLDS), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, cid in (("world_pos", WORLD_POS), ("world_vel", WORLD_VEL), ("world_accel", WORLD_ACCEL), ("force", FORCE)):
+        np.save(os.path.join(out_dir, name + ".npy"), ex.download(cid)[idx])
 
 
 def run_b200(args):
-    ensure_built()
     import torch
     import torch.distributed as dist
 
@@ -409,6 +411,8 @@ def run_b200(args):
         t_end = time.perf_counter()
         ms = max_over_ranks(e0.elapsed_time(e1))
         launches = ex.timings()["kernel_launches"] - launches0
+        if args.dump_outputs and rank == 0:  # the state of the last timed step, before the clock replay below moves it on
+            dump_outputs(ex, args.dump_outputs)
         window = "timed region"
         if ms * 1e-3 < 0.3:  # `ms` is the max over ranks, so every rank takes the same branch
             # too short for nvidia-smi's 50 ms period: replay the identical loop for ~0.5 s and sample that
@@ -932,8 +936,12 @@ def main():
     ap.add_argument("--mc-steps", type=int, default=1000, help="configs[4]: ticks per rollout (dt = 1e-3)")
     ap.add_argument("--configs", action="store_true", help="also time the other BASELINE.json configs (adds ~1 min)")
     ap.add_argument("--kernel-only", action="store_true", help="profiling aid: only the main timed loop (no e2e / cpu / extras)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed executor's final state columns (a fixed sample of "
+                                                            f"{DUMP_WORLDS} worlds) to DIR/<column>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the state of the B200 executor: it needs --impl b200")
         return run_reference(args)
     return run_b200(args)
 
