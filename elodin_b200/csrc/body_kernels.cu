@@ -145,8 +145,14 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_fast_spec_kernel(const __gri
     B200_LDV(P.pos, 4, x[k].x.x); B200_LDV(P.pos, 5, x[k].x.y); B200_LDV(P.pos, 6, x[k].x.z);
     B200_LDV(P.vel, 0, v[k].ang.x); B200_LDV(P.vel, 1, v[k].ang.y); B200_LDV(P.vel, 2, v[k].ang.z);
     B200_LDV(P.vel, 3, v[k].lin.x); B200_LDV(P.vel, 4, v[k].lin.y); B200_LDV(P.vel, 5, v[k].lin.z);
-    // the inertia diagonal only matters to a body-frame torque (or to the Force column written back)
-    { B200_LDV(P.ine, 0, I[k].diag.x); B200_LDV(P.ine, 1, I[k].diag.y); B200_LDV(P.ine, 2, I[k].diag.z); }
+    // the inertia diagonal only matters to invI (a torque) and to the Force column (the launch that writes it back,
+    // 25-plane trajectory samples): every other launch leaves its 24 B per body unread.  The mass always matters.
+    if (sig_needs_invI(SIG) || P.write_fa || (TRAJ && P.traj_planes == 25)) {
+        B200_LDV(P.ine, 0, I[k].diag.x); B200_LDV(P.ine, 1, I[k].diag.y); B200_LDV(P.ine, 2, I[k].diag.z);
+    } else {
+#pragma unroll
+        for (int k = 0; k < BPT; ++k) I[k].diag = Vec3{0.0, 0.0, 0.0};
+    }
     B200_LDV(P.ine, 6, I[k].m);
 #pragma unroll
     for (int k = 0; k < BPT; ++k) {
@@ -182,11 +188,25 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_fast_spec_kernel(const __gri
     // tick of arithmetic later (telemetry on every tick: 254 -> see profiles/r02_tune_telemetry.txt)
     const bool defer_traj = TRAJ && BPT == 2 && both && P.n_ticks == 1 && P.traj_planes == 13;
     Motion a_last[BPT], f_last[BPT];
+    // Force-free tick: every stage acceleration is (0*m)*rcp(m), +-0 for a finite nonzero mass, so the new velocity has
+    // the loaded bits except for a -0 component, a degenerate mass (NaN) or a NaN payload.  Bit j of vdirty: velocity
+    // plane j changed for a body of this thread (compared as integers: +-0 and NaN payloads count).  Planes that did
+    // not change are not stored, and their L2 lines stay clean instead of costing a DRAM write-back.  The pair's
+    // second body outside the range (odd tail) is not integrated, so it never marks a plane.
+    uint32_t vdirty = 0x3fu;
 #pragma unroll
-    for (int k = 0; k < BPT; ++k)
+    for (int k = 0; k < BPT; ++k) {
+        const Motion v_in = v[k];
         if (k == 0 || both)
             fast_ticks<INTEG, TRAJ, false, SIG>(P, b0 + k, x[k], v[k], I[k], a_last[k], f_last[k], P.n_ticks, P.tick0,
                                                 P.write_fa != 0, GravReg{}, in[k], !defer_traj);
+        if (SIG == SIG_FREE) {
+            if (k == 0) vdirty = 0u;
+            auto ne = [](double a, double b) { return (uint32_t)(__double_as_longlong(a) != __double_as_longlong(b)); };
+            vdirty |= ne(v_in.ang.x, v[k].ang.x) | ne(v_in.ang.y, v[k].ang.y) << 1 | ne(v_in.ang.z, v[k].ang.z) << 2 |
+                      ne(v_in.lin.x, v[k].lin.x) << 3 | ne(v_in.lin.y, v[k].lin.y) << 4 | ne(v_in.lin.z, v[k].lin.z) << 5;
+        }
+    }
     if (TRAJ && BPT == 2 && defer_traj && P.traj_every) {
         const uint64_t after = P.tick0 + 1;
         const uint64_t slot = after / P.traj_every - 1;
@@ -203,8 +223,12 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_fast_spec_kernel(const __gri
 
     B200_STV(P.pos, 0, x[k].q.i); B200_STV(P.pos, 1, x[k].q.j); B200_STV(P.pos, 2, x[k].q.k); B200_STV(P.pos, 3, x[k].q.w);
     B200_STV(P.pos, 4, x[k].x.x); B200_STV(P.pos, 5, x[k].x.y); B200_STV(P.pos, 6, x[k].x.z);
-    B200_STV(P.vel, 0, v[k].ang.x); B200_STV(P.vel, 1, v[k].ang.y); B200_STV(P.vel, 2, v[k].ang.z);
-    B200_STV(P.vel, 3, v[k].lin.x); B200_STV(P.vel, 4, v[k].lin.y); B200_STV(P.vel, 5, v[k].lin.z);
+    if (vdirty & 1u) B200_STV(P.vel, 0, v[k].ang.x);
+    if (vdirty & 2u) B200_STV(P.vel, 1, v[k].ang.y);
+    if (vdirty & 4u) B200_STV(P.vel, 2, v[k].ang.z);
+    if (vdirty & 8u) B200_STV(P.vel, 3, v[k].lin.x);
+    if (vdirty & 16u) B200_STV(P.vel, 4, v[k].lin.y);
+    if (vdirty & 32u) B200_STV(P.vel, 5, v[k].lin.z);
     if (P.write_fa) {
         B200_STV(P.acc, 0, a_last[k].ang.x); B200_STV(P.acc, 1, a_last[k].ang.y); B200_STV(P.acc, 2, a_last[k].ang.z);
         B200_STV(P.acc, 3, a_last[k].lin.x); B200_STV(P.acc, 4, a_last[k].lin.y); B200_STV(P.acc, 5, a_last[k].lin.z);
@@ -380,7 +404,8 @@ __global__ void __launch_bounds__(kPipeTB, MINB) body_fast_pipe_kernel(const __g
 // A signature covers an effector list when the folded result does not depend on anything the compile-time form
 // cannot express: no entity masks (query-join membership), at most one thrust / wrench / drag / frame effector,
 // no wrench ahead of the drag (apply_drag resets the torque accumulated before it), a drag that has its wind
-// column, the edge_fold gravity first.  Everything else keeps the run-time interpreter.
+// column, the edge_fold gravity first.  Everything else keeps the run-time interpreter.  A list that applies no force
+// at all (empty, or constant gravities that sum to exactly zero) is SIG_FREE.
 static uint32_t spec_signature(StepParams &Q)
 {
     uint32_t sig = 0;
@@ -444,6 +469,7 @@ static uint32_t spec_signature(StepParams &Q)
         }
     }
     Q.spec = sp;
+    if (sig == 0u && sp.g[0] == 0.0 && sp.g[1] == 0.0 && sp.g[2] == 0.0) return SIG_FREE;
     return sig;
 }
 
@@ -499,10 +525,10 @@ static void launch_spec(const StepParams &Q, cudaStream_t s)
 
 // signatures with a compiled kernel; anything else falls back to the interpreter kernel
 #ifdef B200_TUNE
-#define B200_SPEC_SIGS(X) X(0u) X(SIG_THRUST | SIG_DRAG) X(SIG_FRAME | SIG_WRENCH)
+#define B200_SPEC_SIGS(X) X(SIG_FREE) X(0u) X(SIG_THRUST | SIG_DRAG) X(SIG_FRAME | SIG_WRENCH)
 #else
 #define B200_SPEC_SIGS(X)                                                                                        \
-    X(0u) X(SIG_DRAG) X(SIG_THRUST) X(SIG_WRENCH) X(SIG_FRAME) X(SIG_GRAPH)                                       \
+    X(SIG_FREE) X(0u) X(SIG_DRAG) X(SIG_THRUST) X(SIG_WRENCH) X(SIG_FRAME) X(SIG_GRAPH)                                       \
     X(SIG_THRUST | SIG_DRAG) X(SIG_THRUST | SIG_DRAG | SIG_DRAG_PB) X(SIG_THRUST | SIG_WRENCH) X(SIG_FRAME | SIG_WRENCH)     \
     X(SIG_J2) X(SIG_WHEELS | SIG_J2) X(SIG_WWORLD) X(SIG_WHEELS | SIG_WWORLD)
 #endif

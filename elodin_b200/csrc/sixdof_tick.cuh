@@ -330,8 +330,17 @@ enum : uint32_t {
     SIG_J2 = 64u,             // GRAVITY_J2
     SIG_WHEELS = 128u,        // TORQUE_BODY_FOLD with three wheels (the cube-sat shape), first in the list
     SIG_WWORLD = 256u,        // WRENCH_WORLD: externally computed world-frame wrench column
+    SIG_FREE = 512u,          // no effector and a summed constant gravity of exactly (0, 0, 0).  The tick is the sig-0
+                              // arithmetic unchanged; only the kernel's velocity write-back differs (no effector code
+                              // tests this bit)
     SIG_GENERIC = 0x80000000u // interpret StepParams::eff[] at run time
 };
+
+// The inertia diagonal enters the tick only through invI, which only body-frame and world-frame torques need
+__host__ __device__ constexpr bool sig_needs_invI(uint32_t sig)
+{
+    return sig == SIG_GENERIC || (sig & (SIG_WRENCH | SIG_WHEELS | SIG_WWORLD)) != 0;
+}
 
 // per-body effector inputs of a specialised kernel: loaded next to the state, before any arithmetic
 struct EffIn {
@@ -558,7 +567,7 @@ __device__ __forceinline__ void fast_ticks(const StepParams &P, uint64_t b, Pose
                                            const GravReg &greg, const EffIn &in = EffIn{}, bool store_traj = true)
 {
     constexpr bool GEN = SIG == SIG_GENERIC;
-    constexpr bool NEED_INVI = GEN || (SIG & (SIG_WRENCH | SIG_WHEELS | SIG_WWORLD));
+    constexpr bool NEED_INVI = sig_needs_invI(SIG);
     const Vec3 invI = NEED_INVI ? Vec3{fa::rcp_nr(I.diag.x), fa::rcp_nr(I.diag.y), fa::rcp_nr(I.diag.z)} : Vec3{0.0, 0.0, 0.0};
     const double inv_m = fa::rcp_nr(I.m);
     Folded f;
