@@ -21,8 +21,9 @@ from .effectors import (DragQuadratic, GravityConst, GravityEGM08, GravityEdges,
                         TorqueBodyFold, WrenchBody, WrenchWorld, all_pairs_edges)
 from .executor import B200Exec, device_count, pinned_empty, pinned_free
 from .world import (Annotated, Archetype, Body, Component, ComponentType, Edge, EntityId, Exec, Force, HostSystem,
-                    Inertia, Integrator, PrimitiveType, Quaternion, Seed, SimulationTick, SimulationTimeStep,
+                    Inertia, InputSchedule, Integrator, PrimitiveType, Quaternion, Seed, SimulationTick, SimulationTimeStep,
                     SpatialForce, SpatialInertia, SpatialMotion, SpatialTransform, StepContext, World, WorldAccel,
-                    WorldPos, WorldVel, dataclass, host_system, quantised_time_step, six_dof, ticks_per_telemetry)
+                    WorldPos, WorldVel, dataclass, host_system, input_schedule, quantised_time_step, schedule_row, six_dof,
+                    ticks_per_telemetry)
 
 __all__ = [n for n in dir() if not n.startswith("_")]

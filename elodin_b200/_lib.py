@@ -49,7 +49,8 @@ SYMBOLS = [
     "b200_component_id", "b200_last_error", "b200_device_count", "b200_host_alloc", "b200_host_alloc_local", "b200_host_free",
     "b200_device_numa_node", "b200_host_node_of",
     "b200_sixdof_create", "b200_sixdof_destroy", "b200_sixdof_input_ids", "b200_sixdof_output_ids",
-    "b200_sixdof_column_bytes", "b200_sixdof_upload", "b200_sixdof_download", "b200_sixdof_step",
+    "b200_sixdof_column_bytes", "b200_sixdof_upload", "b200_sixdof_download", "b200_sixdof_set_schedule",
+    "b200_sixdof_clear_schedule", "b200_sixdof_step",
     "b200_sixdof_sync", "b200_sixdof_invoke_batch", "b200_sixdof_bind_tick", "b200_sixdof_tick",
     "b200_sixdof_trajectory_len", "b200_sixdof_trajectory_width", "b200_sixdof_trajectory_download",
     "b200_sixdof_trajectory_reset",
@@ -167,6 +168,8 @@ def lib():
     L.b200_sixdof_column_bytes.restype = u64
     L.b200_sixdof_upload.argtypes = [vp, u64, vp, u64]
     L.b200_sixdof_download.argtypes = [vp, u64, vp, u64]
+    L.b200_sixdof_set_schedule.argtypes = [vp, u64, vp, u64, u64, u64]
+    L.b200_sixdof_clear_schedule.argtypes = [vp, u64]
     L.b200_sixdof_step.argtypes = [vp, u64]
     L.b200_sixdof_sync.argtypes = [vp]
     L.b200_sixdof_invoke_batch.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), u64]

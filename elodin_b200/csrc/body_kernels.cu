@@ -17,7 +17,8 @@ namespace b200 {
 
 // ================================================================== EXACT body kernel
 
-template <int INTEG, int BLOCK, int MINB, bool UNR = false, uint32_t SEQ = SEQ_INTERPRET>
+// SCHED: the launch integrates several ticks of input schedules (P.sched); tick t reads the rows of Tick P.tick_abs + t
+template <int INTEG, int BLOCK, int MINB, bool UNR = false, uint32_t SEQ = SEQ_INTERPRET, bool SCHED = false>
 __global__ void __launch_bounds__(BLOCK, MINB) body_exact_kernel(const __grid_constant__ StepParams P)
 {
     const uint64_t b = (uint64_t)blockIdx.x * BLOCK + threadIdx.x;
@@ -34,7 +35,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_exact_kernel(const __grid_co
     uint64_t traj_slot = 0;
     if (P.traj_every) { traj_phase = (uint32_t)(P.tick0 % P.traj_every); traj_slot = P.tick0 / P.traj_every; }
     for (uint32_t t = 0; t < P.n_ticks; ++t) {
-        exact_tick<INTEG, false, UNR, SEQ>(P, b, x0, v0, a_out, f_out, I, no_greg);
+        exact_tick<INTEG, false, UNR, SEQ, SCHED>(P, b, x0, v0, a_out, f_out, I, no_greg, P.tick_abs + t);
         if (P.traj_every && ++traj_phase == P.traj_every) {
             traj_phase = 0;
             if (traj_slot < P.traj_capacity) {
@@ -67,7 +68,7 @@ __device__ __forceinline__ void prefetch_effector_columns(const StepParams &P, u
         for (uint32_t k = 0; k < 9; ++k) asm volatile("prefetch.global.L1 [%0];" ::"l"(P.gforce + (uint64_t)k * P.ld + b));
 }
 
-template <int INTEG, int BLOCK, int MINB, bool TRAJ>
+template <int INTEG, int BLOCK, int MINB, bool TRAJ, bool SCHED = false>
 __global__ void __launch_bounds__(BLOCK, MINB) body_fast_kernel(const __grid_constant__ StepParams P)
 {
     const uint64_t b = (uint64_t)blockIdx.x * BLOCK + threadIdx.x;
@@ -77,7 +78,7 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_fast_kernel(const __grid_con
     Motion v0 = load_motion(P.vel, P.ld, b);
     const Inertia I = load_inertia(P.ine, P.ld, b);
     Motion a_last, f_last;
-    fast_ticks<INTEG, TRAJ>(P, b, x0, v0, I, a_last, f_last, P.n_ticks, P.tick0, P.write_fa != 0, GravReg{});
+    fast_ticks<INTEG, TRAJ, false, SIG_GENERIC, SCHED>(P, b, x0, v0, I, a_last, f_last, P.n_ticks, P.tick0, P.write_fa != 0, GravReg{});
     store_pose(P.pos, P.ld, b, x0);
     store_motion(P.vel, P.ld, b, v0);
     if (P.write_fa) {
@@ -125,7 +126,9 @@ template <> struct VecIO<2> {
         VecIO<BPT>::st((base) + (uint64_t)(plane) * P.ld, b0, t_, both);                   \
     } while (0)
 
-template <int INTEG, uint32_t SIG, bool TRAJ, int BLOCK, int MINB, int BPT>
+// SCHED: the launch integrates several ticks of input schedules (P.sched): the first tick's inputs load with the state
+// from the rows of Tick P.tick_abs, every later tick reloads its own rows and refolds (fast_ticks)
+template <int INTEG, uint32_t SIG, bool TRAJ, int BLOCK, int MINB, int BPT, bool SCHED = false>
 __global__ void __launch_bounds__(BLOCK, MINB) body_fast_spec_kernel(const __grid_constant__ StepParams P)
 {
     // Odd launches walk the planes from the far end: the tail of the state the previous launch read and wrote last is
@@ -159,28 +162,39 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_fast_spec_kernel(const __gri
         in[k].thrust = 0.0; in[k].cd_rho = in[k].area = 0.0;
         in[k].wr_t = in[k].wr_f = in[k].wind = in[k].wheels = in[k].ww_t = in[k].ww_f = Vec3{0.0, 0.0, 0.0};
     }
-    if (SIG & SIG_THRUST) B200_LDV(P.spec.thrust, 0, in[k].thrust);
+    // input columns; a scheduled launch reads the rows of its first tick here
+    const double *c_thrust = P.spec.thrust, *c_wr_t = P.spec.wr_t, *c_wr_f = P.spec.wr_f, *c_wheels = P.spec.wheels,
+                 *c_wworld = P.spec.wworld, *c_drag = P.spec.drag;
+    if constexpr (SCHED) {
+        c_thrust = schedule_ptr(c_thrust, P.spec.s_thrust, P.tick_abs);
+        c_wr_t = schedule_ptr(c_wr_t, P.spec.s_wrench, P.tick_abs);
+        c_wr_f = schedule_ptr(c_wr_f, P.spec.s_wrench, P.tick_abs);
+        c_wheels = schedule_ptr(c_wheels, P.spec.s_wheels, P.tick_abs);
+        c_wworld = schedule_ptr(c_wworld, P.spec.s_wworld, P.tick_abs);
+        c_drag = schedule_ptr(c_drag, P.spec.s_drag, P.tick_abs);
+    }
+    if (SIG & SIG_THRUST) B200_LDV(c_thrust, 0, in[k].thrust);
     if (SIG & SIG_WRENCH) {
-        B200_LDV(P.spec.wr_t, 0, in[k].wr_t.x); B200_LDV(P.spec.wr_t, 1, in[k].wr_t.y); B200_LDV(P.spec.wr_t, 2, in[k].wr_t.z);
-        B200_LDV(P.spec.wr_f, 0, in[k].wr_f.x); B200_LDV(P.spec.wr_f, 1, in[k].wr_f.y); B200_LDV(P.spec.wr_f, 2, in[k].wr_f.z);
+        B200_LDV(c_wr_t, 0, in[k].wr_t.x); B200_LDV(c_wr_t, 1, in[k].wr_t.y); B200_LDV(c_wr_t, 2, in[k].wr_t.z);
+        B200_LDV(c_wr_f, 0, in[k].wr_f.x); B200_LDV(c_wr_f, 1, in[k].wr_f.y); B200_LDV(c_wr_f, 2, in[k].wr_f.z);
     }
     if (SIG & SIG_WHEELS) { // the three wheel torques only ever enter as their sum (the rotation is linear)
         Vec3 w[BPT][3];
 #pragma unroll
         for (int q = 0; q < 3; ++q) {
-            B200_LDV(P.spec.wheels, 3 * q + 0, w[k][q].x); B200_LDV(P.spec.wheels, 3 * q + 1, w[k][q].y); B200_LDV(P.spec.wheels, 3 * q + 2, w[k][q].z);
+            B200_LDV(c_wheels, 3 * q + 0, w[k][q].x); B200_LDV(c_wheels, 3 * q + 1, w[k][q].y); B200_LDV(c_wheels, 3 * q + 2, w[k][q].z);
         }
 #pragma unroll
         for (int k = 0; k < BPT; ++k)
             in[k].wheels = Vec3{w[k][0].x + w[k][1].x + w[k][2].x, w[k][0].y + w[k][1].y + w[k][2].y, w[k][0].z + w[k][1].z + w[k][2].z};
     }
     if (SIG & SIG_WWORLD) {
-        B200_LDV(P.spec.wworld, 0, in[k].ww_t.x); B200_LDV(P.spec.wworld, 1, in[k].ww_t.y); B200_LDV(P.spec.wworld, 2, in[k].ww_t.z);
-        B200_LDV(P.spec.wworld, 3, in[k].ww_f.x); B200_LDV(P.spec.wworld, 4, in[k].ww_f.y); B200_LDV(P.spec.wworld, 5, in[k].ww_f.z);
+        B200_LDV(c_wworld, 0, in[k].ww_t.x); B200_LDV(c_wworld, 1, in[k].ww_t.y); B200_LDV(c_wworld, 2, in[k].ww_t.z);
+        B200_LDV(c_wworld, 3, in[k].ww_f.x); B200_LDV(c_wworld, 4, in[k].ww_f.y); B200_LDV(c_wworld, 5, in[k].ww_f.z);
     }
     if (SIG & SIG_DRAG) {
-        B200_LDV(P.spec.drag, 0, in[k].wind.x); B200_LDV(P.spec.drag, 1, in[k].wind.y); B200_LDV(P.spec.drag, 2, in[k].wind.z);
-        if (SIG & SIG_DRAG_PB) { B200_LDV(P.spec.drag, 3, in[k].cd_rho); B200_LDV(P.spec.drag, 4, in[k].area); }
+        B200_LDV(c_drag, 0, in[k].wind.x); B200_LDV(c_drag, 1, in[k].wind.y); B200_LDV(c_drag, 2, in[k].wind.z);
+        if (SIG & SIG_DRAG_PB) { B200_LDV(c_drag, 3, in[k].cd_rho); B200_LDV(c_drag, 4, in[k].area); }
     }
 
     // A (WorldPos, WorldVel) sample on every launch of one tick: the pair stores it from here as one 16-byte store per
@@ -198,8 +212,8 @@ __global__ void __launch_bounds__(BLOCK, MINB) body_fast_spec_kernel(const __gri
     for (int k = 0; k < BPT; ++k) {
         const Motion v_in = v[k];
         if (k == 0 || both)
-            fast_ticks<INTEG, TRAJ, false, SIG>(P, b0 + k, x[k], v[k], I[k], a_last[k], f_last[k], P.n_ticks, P.tick0,
-                                                P.write_fa != 0, GravReg{}, in[k], !defer_traj);
+            fast_ticks<INTEG, TRAJ, false, SIG, SCHED>(P, b0 + k, x[k], v[k], I[k], a_last[k], f_last[k], P.n_ticks, P.tick0,
+                                                       P.write_fa != 0, GravReg{}, in[k], !defer_traj);
         if (SIG == SIG_FREE) {
             if (k == 0) vdirty = 0u;
             auto ne = [](double a, double b) { return (uint32_t)(__double_as_longlong(a) != __double_as_longlong(b)); };
@@ -424,12 +438,14 @@ static uint32_t spec_signature(StepParams &Q)
             sig |= SIG_DRAG | (E.col_width == 5 ? SIG_DRAG_PB : 0u);
             sp.kd = 0.5 * E.p[0] * E.p[1];
             sp.drag = E.col;
+            sp.s_drag = E.sched;
             break;
         case B200_EFF_THRUST_BODY:
             if (!E.col || ++n_thrust > 1) return SIG_GENERIC;
             sig |= SIG_THRUST;
             sp.axis[0] = E.p[0]; sp.axis[1] = E.p[1]; sp.axis[2] = E.p[2];
             sp.thrust = E.col;
+            sp.s_thrust = E.sched;
             break;
         case B200_EFF_WRENCH_BODY: {
             if (!E.col || ++n_wrench > 1) return SIG_GENERIC;
@@ -438,6 +454,7 @@ static uint32_t spec_signature(StepParams &Q)
             const uint64_t to = (E.flags & B200_EFF_FLAG_WRENCH_LINEAR_FIRST) ? 3 : 0;
             sp.wr_t = E.col + to * Q.ld;
             sp.wr_f = E.col + (3 - to) * Q.ld;
+            sp.s_wrench = E.sched;
             break;
         }
         case B200_EFF_GRAVITY_FRAME:
@@ -459,11 +476,13 @@ static uint32_t spec_signature(StepParams &Q)
             if (!E.col || (sig & SIG_WWORLD)) return SIG_GENERIC;
             sig |= SIG_WWORLD;
             sp.wworld = E.col;
+            sp.s_wworld = E.sched;
             break;
         case B200_EFF_TORQUE_BODY_FOLD: // the fold overwrites Force: only as the first effector is it a plain torque term
             if (i != 0 || !E.col || E.col_width != 9) return SIG_GENERIC;
             sig |= SIG_WHEELS;
             sp.wheels = E.col;
+            sp.s_wheels = E.sched;
             break;
         default: return SIG_GENERIC;
         }
@@ -475,12 +494,12 @@ static uint32_t spec_signature(StepParams &Q)
 
 // launch shape of the specialised kernels: (threads per CTA, resident CTAs per SM the register allocation is bounded
 // for, bodies per thread).  B200_SPEC_CFG selects among the shapes a tuning build (-DB200_TUNE) instantiates.
-template <int INTEG, uint32_t SIG, bool TRAJ, int BLOCK, int MINB, int BPT>
+template <int INTEG, uint32_t SIG, bool TRAJ, int BLOCK, int MINB, int BPT, bool SCHED = false>
 static void launch_spec_shape(const StepParams &Q, cudaStream_t s)
 {
     const uint64_t threads = (Q.n_bodies + BPT - 1) / BPT;
     const unsigned grid = (unsigned)((threads + BLOCK - 1) / BLOCK);
-    body_fast_spec_kernel<INTEG, SIG, TRAJ, BLOCK, MINB, BPT><<<grid, BLOCK, 0, s>>>(Q);
+    body_fast_spec_kernel<INTEG, SIG, TRAJ, BLOCK, MINB, BPT, SCHED><<<grid, BLOCK, 0, s>>>(Q);
 }
 
 static bool planes_16B_aligned(const StepParams &Q, uint32_t sig)
@@ -491,7 +510,10 @@ static bool planes_16B_aligned(const StepParams &Q, uint32_t sig)
     if (sig & SIG_DRAG) a |= (uintptr_t)Q.spec.drag;
     if (sig & SIG_WHEELS) a |= (uintptr_t)Q.spec.wheels;
     if (sig & SIG_WWORLD) a |= (uintptr_t)Q.spec.wworld;
-    return (a & 15u) == 0 && (Q.ld & 1u) == 0;
+    // every row of a scheduled column starts a whole number of rows (width * ld doubles) after the table base
+    const uint64_t strides = Q.spec.s_thrust.stride | Q.spec.s_wrench.stride | Q.spec.s_drag.stride | Q.spec.s_wheels.stride |
+                             Q.spec.s_wworld.stride;
+    return (a & 15u) == 0 && (Q.ld & 1u) == 0 && (strides & 1u) == 0;
 }
 
 // Default shape, measured on B200 at 2^22 worlds (profiles/r02_tune_spec.md): body pairs (BPT = 2, LDG.E.128) at
@@ -499,10 +521,16 @@ static bool planes_16B_aligned(const StepParams &Q, uint32_t sig)
 // algorithmic bytes; one body per thread at 128 x 4 is 9 % (rocket) to 11 % (falcon9) slower.  Ranges too small to
 // fill the machine with pairs, or whose planes are not 16-byte aligned (odd world-range offsets), take one body
 // per thread.
-template <int INTEG, uint32_t SIG, bool TRAJ>
+template <int INTEG, uint32_t SIG, bool TRAJ, bool SCHED = false>
 static void launch_spec(const StepParams &Q, cudaStream_t s)
 {
     const bool vec_ok = planes_16B_aligned(Q, SIG);
+    if constexpr (SCHED) { // the default shapes only
+        constexpr uint64_t kPairMinBodies = 2ull * 128 * 3 * 148;
+        if (vec_ok && Q.n_bodies >= kPairMinBodies) launch_spec_shape<INTEG, SIG, TRAJ, 128, 3, 2, true>(Q, s);
+        else launch_spec_shape<INTEG, SIG, TRAJ, 128, 4, 1, true>(Q, s);
+        return;
+    }
 #ifdef B200_TUNE
     const int cfg = env_int("B200_SPEC_CFG", -1); // re-read per launch: one tuning process sweeps the shapes
     switch (cfg) {
@@ -533,10 +561,31 @@ static void launch_spec(const StepParams &Q, cudaStream_t s)
     X(SIG_J2) X(SIG_WHEELS | SIG_J2) X(SIG_WWORLD) X(SIG_WHEELS | SIG_WWORLD)
 #endif
 
+// the signatures that read an input column, compiled a second time for fused launches with input schedules
+#ifdef B200_TUNE
+#define B200_SCHED_SIGS(X) X(SIG_THRUST | SIG_DRAG)
+#else
+#define B200_SCHED_SIGS(X)                                                                                                 \
+    X(SIG_DRAG) X(SIG_THRUST) X(SIG_WRENCH) X(SIG_THRUST | SIG_DRAG) X(SIG_THRUST | SIG_DRAG | SIG_DRAG_PB)                \
+    X(SIG_THRUST | SIG_WRENCH) X(SIG_FRAME | SIG_WRENCH) X(SIG_WHEELS | SIG_J2) X(SIG_WWORLD) X(SIG_WHEELS | SIG_WWORLD)
+#endif
+
 template <int INTEG>
 static bool launch_spec_sig(const StepParams &Q, uint32_t sig, cudaStream_t s)
 {
     const bool traj = Q.traj_every != 0;
+    if (Q.sched) {
+        switch (sig) {
+#define X(SIGV)                                                                \
+    case (SIGV):                                                               \
+        if (traj) launch_spec<INTEG, (SIGV), true, true>(Q, s);                \
+        else launch_spec<INTEG, (SIGV), false, true>(Q, s);                    \
+        return true;
+            B200_SCHED_SIGS(X)
+#undef X
+        default: return false;
+        }
+    }
     switch (sig) {
 #define X(SIGV)                                                                \
     case (SIGV):                                                               \
@@ -575,6 +624,29 @@ static uint32_t exact_sequence(const StepParams &P)
     return seq;
 }
 
+// the sequences that read an input column, compiled a second time for fused launches with input schedules
+#define B200_EXACT_SCHED_SEQS(X)                                                                                        \
+    X(B200_SEQ2(B200_EFF_GRAVITY_CONST, B200_EFF_DRAG_QUADRATIC))                                                       \
+    X(B200_SEQ3(B200_EFF_GRAVITY_CONST, B200_EFF_THRUST_BODY, B200_EFF_DRAG_QUADRATIC))                                 \
+    X(B200_SEQ3(B200_EFF_GRAVITY_CONST, B200_EFF_THRUST_BODY, B200_EFF_WRENCH_BODY))                                    \
+    X(B200_SEQ2(B200_EFF_GRAVITY_FRAME, B200_EFF_WRENCH_BODY))                                                          \
+    X(B200_SEQ2(B200_EFF_TORQUE_BODY_FOLD, B200_EFF_WRENCH_WORLD))
+
+template <int INTEG, int BLOCK, int MINB>
+static bool launch_exact_sched(const StepParams &P, uint32_t seq, cudaStream_t s)
+{
+    const unsigned grid = (unsigned)((P.n_bodies + BLOCK - 1) / BLOCK);
+    switch (seq) {
+#define X(SEQV)                                                                            \
+    case (SEQV):                                                                           \
+        body_exact_kernel<INTEG, BLOCK, MINB, false, (SEQV), true><<<grid, BLOCK, 0, s>>>(P); \
+        return true;
+        B200_EXACT_SCHED_SEQS(X)
+#undef X
+    default: body_exact_kernel<INTEG, BLOCK, MINB, false, SEQ_INTERPRET, true><<<grid, BLOCK, 0, s>>>(P); return true;
+    }
+}
+
 template <int INTEG, int BLOCK, int MINB>
 static bool launch_exact_seq(const StepParams &P, uint32_t seq, cudaStream_t s)
 {
@@ -594,6 +666,31 @@ cudaError_t launch_body_step(const StepParams &P, int integrator, int math_mode,
 {
     if (P.n_bodies == 0) return cudaSuccess;
     const bool rk4 = integrator == B200_INTEGRATOR_RK4;
+    if (P.sched) {
+        // several ticks of input schedules in one launch: the kernels compiled to read each tick's rows, in the default
+        // shapes (the tuning switches below do not apply)
+        if (math_mode == B200_MATH_EXACT) {
+            const uint32_t seq = exact_sequence(P);
+            if (rk4) launch_exact_sched<B200_INTEGRATOR_RK4, 128, 4>(P, seq, s);
+            else launch_exact_sched<B200_INTEGRATOR_SEMI_IMPLICIT, 256, 1>(P, seq, s);
+            return cudaGetLastError();
+        }
+        StepParams Q = P;
+        const uint32_t sig = spec_signature(Q);
+        const bool done = sig != SIG_GENERIC && (rk4 ? launch_spec_sig<B200_INTEGRATOR_RK4>(Q, sig, s)
+                                                     : launch_spec_sig<B200_INTEGRATOR_SEMI_IMPLICIT>(Q, sig, s));
+        if (!done) {
+            auto g = [&](int blk) { return (unsigned)((P.n_bodies + blk - 1) / blk); };
+            if (rk4) {
+                if (P.traj_every) body_fast_kernel<B200_INTEGRATOR_RK4, 128, 4, true, true><<<g(128), 128, 0, s>>>(P);
+                else body_fast_kernel<B200_INTEGRATOR_RK4, 128, 4, false, true><<<g(128), 128, 0, s>>>(P);
+            } else {
+                if (P.traj_every) body_fast_kernel<B200_INTEGRATOR_SEMI_IMPLICIT, 128, 4, true, true><<<g(128), 128, 0, s>>>(P);
+                else body_fast_kernel<B200_INTEGRATOR_SEMI_IMPLICIT, 128, 4, false, true><<<g(128), 128, 0, s>>>(P);
+            }
+        }
+        return cudaGetLastError();
+    }
     if (math_mode == B200_MATH_EXACT) {
 #ifdef B200_TUNE
         const int xcfg = env_int("B200_EXACT_CFG", 3);

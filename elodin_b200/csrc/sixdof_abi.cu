@@ -240,6 +240,54 @@ void fill_step_params(b200_sixdof *h, StepParams &P)
 
 namespace {
 
+bool is_state_column(uint64_t id)
+{
+    return id == B200_ID_WORLD_POS || id == B200_ID_WORLD_VEL || id == B200_ID_WORLD_ACCEL || id == B200_ID_FORCE ||
+           id == B200_ID_INERTIA || id == B200_ID_TICK || id == B200_ID_SIMULATION_TIME_STEP;
+}
+
+// Point every scheduled effector column of a launch of n ticks, the first of which has Tick value `tick`, at its
+// table.  One tick reads one fixed row: the kernels see a plain column and every existing instantiation applies.
+// Several ticks carry the row stride and the row rule; the kernels compiled for it read each tick's own row.
+void bind_schedules(b200_sixdof *h, StepParams &P, uint64_t b0, uint64_t n, uint64_t tick)
+{
+    P.tick_abs = tick;
+    P.sched = 0;
+    if (h->schedules.empty()) return;
+    for (uint32_t i = 0; i < P.n_eff; ++i) {
+        const uint64_t id = h->effectors[i].column_id;
+        const Schedule *s = id ? h->find_schedule(id) : nullptr;
+        if (!s) continue;
+        const uint64_t stride = (uint64_t)s->width * h->ld;
+        if (n == 1) {
+            P.eff[i].col = s->table + schedule_row(tick, s->first_tick, s->n_rows) * stride + b0;
+            P.eff[i].sched = SchedDev{0, 0, 0};
+        } else {
+            P.eff[i].col = s->table + b0;
+            P.eff[i].sched = SchedDev{stride, s->n_rows, s->first_tick};
+            P.sched = 1;
+        }
+    }
+}
+
+// After n ticks the scheduled columns read back as the row of the last one; the copy waits until someone reads them
+void note_schedule_ticks(b200_sixdof *h, uint64_t n_ticks)
+{
+    if (n_ticks == 0) return;
+    for (auto &s : h->schedules) { s.pending = true; s.last_tick = h->tick - 1; }
+}
+
+int materialise_schedule(b200_sixdof *h, Schedule &s)
+{
+    if (!s.pending) return B200_OK;
+    const uint64_t stride = (uint64_t)s.width * h->ld;
+    if (h->n_bodies)
+        CU(h, cudaMemcpyAsync(h->find(s.id)->dev, s.table + schedule_row(s.last_tick, s.first_tick, s.n_rows) * stride,
+                              stride * 8ull, cudaMemcpyDeviceToDevice, h->stream));
+    s.pending = false;
+    return B200_OK;
+}
+
 // Integrate n_ticks ticks of the worlds [w0, w0+nw) on `stream`.  Worlds are independent, so a
 // world range can run to completion before the next one starts (used by the pipelined
 // invoke_batch); counters are the caller's business.
@@ -265,6 +313,7 @@ int launch_ticks(b200_sixdof *h, uint64_t w0, uint64_t nw, uint64_t n_ticks, cud
     double *pos_next = h->pos_alt ? h->pos_alt + b0 : nullptr, *vel_next = h->vel_alt ? h->vel_alt + b0 : nullptr;
     while (left) {
         const uint64_t n = std::min(left, fuse);
+        bind_schedules(h, P, b0, n, h->tick + done);
         if (egm) {
             const b200_effector &ge = h->effectors[h->egm_eff];
             EgmParams E{};
@@ -339,6 +388,7 @@ int do_step(b200_sixdof *h, uint64_t n_ticks)
     h->ticks_done += n_ticks;
     h->tick += n_ticks;
     h->timings.ticks += n_ticks;
+    note_schedule_ticks(h, n_ticks);
     return B200_OK;
 }
 
@@ -350,6 +400,9 @@ int do_upload(b200_sixdof *h, uint64_t id, const void *src, uint64_t bytes)
         return fail(B200_ERR_VALUE_SIZE_MISMATCH, "component value had wrong size: 0x%016llx has %llu bytes, got %llu",
                     (unsigned long long)id, (unsigned long long)column_bytes(h, *c), (unsigned long long)bytes);
     if (!src) return fail(B200_ERR_INVALID_ARGUMENT, "null source buffer");
+    if (h->find_schedule(id))
+        return fail(B200_ERR_INVALID_ARGUMENT, "column 0x%016llx is driven by an input schedule (clear it to upload)",
+                    (unsigned long long)id);
     if (c->global) {
         // the two globals are 8-byte host scalars (Globals entity, world.rs:174-191)
         uint64_t raw;
@@ -383,8 +436,9 @@ int do_download(b200_sixdof *h, uint64_t id, void *dst, uint64_t bytes)
         return B200_OK;
     }
     if (bytes == 0) return B200_OK;
-    int rc = ensure_staging(h, bytes);
-    if (rc) return rc;
+    int rc = B200_OK;
+    if (Schedule *s = h->find_schedule(id)) if ((rc = materialise_schedule(h, *s))) return rc;
+    if ((rc = ensure_staging(h, bytes))) return rc;
     CU(h, launch_soa_to_aos(c->dev, h->staging, h->n_bodies, c->width, h->ld, h->stream));
     h->timings.kernel_launches++;
     CU(h, cudaMemcpyAsync(dst, h->staging, bytes, cudaMemcpyDefault, h->stream));
@@ -685,6 +739,7 @@ void b200_sixdof_destroy(b200_sixdof *h)
     if (h->stream) cudaStreamSynchronize(h->stream);
     for (auto &c : h->cols) if (c.dev) cudaFree(c.dev);
     for (auto m : h->eff_masks) if (m) cudaFree(m);
+    for (auto &s : h->schedules) if (s.table) cudaFree(s.table);
     for (auto t : h->eff_tables) if (t) cudaFree(t);
     if (h->row_ptr) cudaFree(h->row_ptr);
     if (h->col_idx) cudaFree(h->col_idx);
@@ -741,6 +796,82 @@ int b200_sixdof_download(b200_sixdof *h, uint64_t id, void *dst, uint64_t bytes)
     if (!h) return fail(B200_ERR_INVALID_ARGUMENT, "null handle");
     CU(h, cudaSetDevice(h->device));
     return do_download(h, id, dst, bytes);
+}
+
+int b200_sixdof_set_schedule(b200_sixdof *h, uint64_t component_id, const void *rows, uint64_t bytes, uint64_t n_rows,
+                             uint64_t first_tick)
+{
+    if (!h) return fail(B200_ERR_INVALID_ARGUMENT, "null handle");
+    if (h->status != B200_OK) return fail(h->status, "handle is in a failed state");
+    CU(h, cudaSetDevice(h->device));
+    Column *c = h->find(component_id);
+    if (!c) return fail(B200_ERR_COMPONENT_NOT_FOUND, "component not found: 0x%016llx", (unsigned long long)component_id);
+    if (is_state_column(component_id))
+        return fail(B200_ERR_INVALID_ARGUMENT, "column 0x%016llx is not an effector input: only effector input columns take a schedule",
+                    (unsigned long long)component_id);
+    if (h->graph_eff >= 0)
+        return fail(B200_ERR_UNSUPPORTED, "input schedules are not supported on graph worlds (edge_fold gravity: small_world_kernel, "
+                                          "nbody_tick_fused_kernel, graph_dense_world_kernel, the graph-force launch)");
+    if (n_rows == 0) return fail(B200_ERR_INVALID_ARGUMENT, "an input schedule needs at least one row");
+    const uint64_t row_bytes = column_bytes(h, *c);
+    if (bytes != n_rows * row_bytes || (row_bytes && bytes / row_bytes != n_rows))
+        return fail(B200_ERR_VALUE_SIZE_MISMATCH, "schedule of 0x%016llx: %llu rows of %llu bytes, got %llu bytes",
+                    (unsigned long long)component_id, (unsigned long long)n_rows, (unsigned long long)row_bytes,
+                    (unsigned long long)bytes);
+    if (bytes && !rows) return fail(B200_ERR_INVALID_ARGUMENT, "null rows buffer");
+    Schedule *old = h->find_schedule(component_id);
+    int rc = B200_OK;
+    if (old && (rc = materialise_schedule(h, *old))) return rc; // the column keeps the row the old schedule last used
+    // device table: row r, plane p at table + (r*width + p)*ld, copied through the staging buffer a few rows at a time
+    const uint64_t stride = (uint64_t)c->width * h->ld;
+    double *table = nullptr;
+    if (h->n_bodies) {
+        if (cudaMalloc(&table, n_rows * stride * 8ull) != cudaSuccess) {
+            (void)cudaGetLastError();
+            return fail(B200_ERR_OUT_OF_MEMORY, "out of device memory for a schedule of %llu rows (%llu bytes)", (unsigned long long)n_rows,
+                        (unsigned long long)(n_rows * stride * 8ull));
+        }
+        auto bail = [&](int code) { cudaFree(table); return code; };
+        if (cudaMemsetAsync(table, 0, n_rows * stride * 8ull, h->stream) != cudaSuccess)
+            return bail(cuda_fail(h, cudaGetLastError(), "cudaMemsetAsync(schedule)"));
+        const uint64_t chunk_rows = std::max<uint64_t>(1, std::min<uint64_t>(n_rows, (64ull << 20) / row_bytes));
+        if ((rc = ensure_staging(h, chunk_rows * row_bytes))) return bail(rc);
+        for (uint64_t r0 = 0; r0 < n_rows; r0 += chunk_rows) {
+            const uint64_t nr = std::min(chunk_rows, n_rows - r0);
+            cudaError_t e = cudaMemcpyAsync(h->staging, (const char *)rows + r0 * row_bytes, nr * row_bytes, cudaMemcpyDefault, h->stream);
+            for (uint64_t r = 0; r < nr && e == cudaSuccess; ++r) {
+                e = launch_aos_to_soa(h->staging + r * (row_bytes / 8), table + (r0 + r) * stride, h->n_bodies, c->width, h->ld, h->stream);
+                h->timings.kernel_launches++;
+            }
+            if (e != cudaSuccess) return bail(cuda_fail(h, e, "schedule upload"));
+        }
+        // the caller's buffer is only valid for this call, and the table an old schedule leaves may still be in use
+        if (cudaStreamSynchronize(h->stream) != cudaSuccess) return bail(cuda_fail(h, cudaGetLastError(), "schedule upload sync"));
+    }
+    if (old) {
+        if (old->table) cudaFree(old->table);
+        old->table = table; old->n_rows = n_rows; old->first_tick = first_tick; old->pending = false;
+    } else {
+        Schedule s{};
+        s.id = component_id; s.width = c->width; s.table = table; s.n_rows = n_rows; s.first_tick = first_tick;
+        h->schedules.push_back(s);
+    }
+    return B200_OK;
+}
+
+int b200_sixdof_clear_schedule(b200_sixdof *h, uint64_t component_id)
+{
+    if (!h) return fail(B200_ERR_INVALID_ARGUMENT, "null handle");
+    CU(h, cudaSetDevice(h->device));
+    if (!h->find(component_id)) return fail(B200_ERR_COMPONENT_NOT_FOUND, "component not found: 0x%016llx", (unsigned long long)component_id);
+    Schedule *s = h->find_schedule(component_id);
+    if (!s) return B200_OK; // nothing bound: the column already drives its effector
+    int rc = materialise_schedule(h, *s); // the column keeps the row its last tick used
+    if (rc) return rc;
+    CU(h, cudaStreamSynchronize(h->stream));
+    if (s->table) cudaFree(s->table);
+    h->schedules.erase(h->schedules.begin() + (s - h->schedules.data()));
+    return B200_OK;
 }
 
 int b200_sixdof_step(b200_sixdof *h, uint64_t n_ticks)
@@ -828,6 +959,7 @@ static int invoke_small(b200_sixdof *h, const uint8_t *const *in_cols, uint8_t *
     h->ticks_done += n_ticks;
     h->tick += n_ticks;
     h->timings.ticks += n_ticks;
+    note_schedule_ticks(h, n_ticks);
     if (out_total) {
         CU(h, launch_multi_transpose(mo, h->n_bodies, h->ld, false, h->stream));
         h->timings.kernel_launches++;
@@ -996,6 +1128,7 @@ static int invoke_pipelined(b200_sixdof *h, const uint8_t *const *in_cols, uint8
     h->ticks_done += n_ticks;
     h->tick += n_ticks;
     h->timings.ticks += n_ticks;
+    note_schedule_ticks(h, n_ticks);
     for (size_t i = 0; i < h->output_ids.size(); ++i) {
         const Column *c = h->find(h->output_ids[i]);
         if (c->global && out_cols[i]) { int rc = do_download(h, c->id, out_cols[i], 8); if (rc) return rc; }
@@ -1034,6 +1167,10 @@ int b200_sixdof_invoke_batch(b200_sixdof *h, const uint8_t *const *in_cols, uint
     // A NULL in_cols[i] means "not dirty" (World::dirty_components, world.rs:43,249-252): the device-resident copy of
     // that column stands.  A NULL out_cols[j] means the caller does not read that column after this batch.
     n_ticks = std::max<uint64_t>(n_ticks, 1); // `n.max(1)`, cranelift_exec.rs:135
+    for (size_t i = 0; i < h->input_ids.size(); ++i)
+        if (in_cols[i] && h->find_schedule(h->input_ids[i]))
+            return fail(B200_ERR_INVALID_ARGUMENT, "input column 0x%016llx is driven by an input schedule: pass NULL for it",
+                        (unsigned long long)h->input_ids[i]);
 
     // World ranges of ~kChunkBodies bodies: range k's PCIe download overlaps range k+1's upload
     // and ticks (two copy engines + the compute stream).  Small batches run as one range.

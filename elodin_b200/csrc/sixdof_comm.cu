@@ -455,6 +455,8 @@ int b200_sixdof_step_row_sharded(b200_sixdof *h, b200_comm *c, uint64_t n_ticks)
 {
     if (!h || !c) return fail(B200_ERR_INVALID_ARGUMENT, "null argument");
     if (h->status != B200_OK) return fail(h->status, "handle is in a failed state");
+    if (!h->schedules.empty())
+        return fail(B200_ERR_UNSUPPORTED, "b200_sixdof_step_row_sharded does not support input schedules (clear them first)");
     if (h->device != c->device) return fail(B200_ERR_INVALID_ARGUMENT, "handle is on device %d, communicator on %d", h->device, c->device);
     if (h->graph_eff < 0 || !h->graph_dense || h->desc.n_worlds != 1 || h->egm_eff >= 0)
         return fail(B200_ERR_UNSUPPORTED, "row sharding applies to one world with dense (all-pairs) edge_fold gravity (and no EGM08 effector)");

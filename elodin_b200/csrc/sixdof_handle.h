@@ -22,6 +22,17 @@ struct Column {
 
 inline uint64_t round_up(uint64_t x, uint64_t m) { return (x + m - 1) / m * m; }
 
+// A per-tick input table bound to one effector input column (b200_sixdof_set_schedule).  Row r, plane p lives at
+// table + (r*width + p)*ld: every row is laid out like the column itself.
+struct Schedule {
+    uint64_t id;
+    uint32_t width;
+    double *table;
+    uint64_t n_rows, first_tick;
+    bool pending = false; // ticks ran since the column last received a row: it still holds an older value
+    uint64_t last_tick = 0; // Tick value of the last integrated tick (the row the column reads back as)
+};
+
 } // namespace b200
 
 struct b200_sixdof {
@@ -36,6 +47,7 @@ struct b200_sixdof {
     uint64_t n_bodies = 0;
     uint64_t ld = 0;
     std::vector<b200::Column> cols;
+    std::vector<b200::Schedule> schedules; // input schedules, at most one per effector input column
     std::vector<uint64_t> input_ids, output_ids;
     double sim_time_step = 0.0;   // SimulationTimeStep column value
     uint64_t tick = 0;            // Tick column value
@@ -79,6 +91,11 @@ struct b200_sixdof {
     const b200::Column *find(uint64_t id) const
     {
         for (auto &c : cols) if (c.id == id) return &c;
+        return nullptr;
+    }
+    b200::Schedule *find_schedule(uint64_t id)
+    {
+        for (auto &s : schedules) if (s.id == id) return &s;
         return nullptr;
     }
 };

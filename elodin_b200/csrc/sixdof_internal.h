@@ -8,6 +8,26 @@
 
 namespace b200 {
 
+// Row of an input schedule (b200_sixdof_set_schedule) that the tick whose Tick column value is `tick` reads: the
+// first row before the table starts, the last one after it ends.  The one place the rule lives (host and device).
+__host__ __device__ __forceinline__ uint64_t schedule_row(uint64_t tick, uint64_t first_tick, uint64_t n_rows)
+{
+    const uint64_t r = tick > first_tick ? tick - first_tick : 0;
+    return r < n_rows ? r : n_rows - 1;
+}
+
+// A scheduled column as a fused launch sees it: row r of the table starts `stride` doubles after row r-1 (width*ld,
+// each row laid out like the column itself); stride 0 = not scheduled, the base is the column (or one fixed row).
+struct SchedDev {
+    uint64_t stride;
+    uint64_t n_rows;
+    uint64_t first_tick;
+};
+__host__ __device__ __forceinline__ const double *schedule_ptr(const double *base, const SchedDev &s, uint64_t tick)
+{
+    return s.stride ? base + schedule_row(tick, s.first_tick, s.n_rows) * s.stride : base;
+}
+
 // One built-in effector as the kernels see it.  `col` points at the SoA planes
 // of its per-body input column (plane p at col + p*ld), nullptr if none.
 struct EffDev {
@@ -19,6 +39,7 @@ struct EffDev {
     uint32_t pad;
     const uint8_t *mask; // [n_entities] or nullptr (query-join membership)
     const double *table; // GRAVITY_EGM08: the term stream sixdof_abi.cu:egm08_tables builds (device)
+    SchedDev sched;      // fused launches of a scheduled column: `col` is the table, tick t reads its row
 };
 
 // Launch parameters of the per-body integrator kernels.  All columns are SoA:
@@ -61,8 +82,12 @@ struct StepParams {
         const double *thrust;        // 1 plane
         const double *wr_t, *wr_f;   // 3 planes each: body-frame torque / force of the wrench column
         const double *drag;          // wind(3) [+ Cd*rho, area]
+        SchedDev s_wheels, s_wworld, s_thrust, s_wrench, s_drag; // the schedules of those columns (stride 0: none)
     } spec;
     EffDev eff[B200_MAX_EFFECTORS];
+    uint64_t tick_abs;  // Tick column value of this launch's first tick (input schedules; tick0 restarts at a trajectory reset)
+    uint32_t sched;     // some eff[].sched is live: the launch integrates > 1 tick and each tick reads its own row
+    uint32_t pad_sched;
 };
 
 // Launch parameters of the edge_fold gravity kernels.

@@ -118,12 +118,15 @@ static __device__ __noinline__ Vec3 j2_field_exact(double mu, double J2, double 
 // clear_forces | effectors (array order) on the stage state; six_dof.rs:148-150,195
 // One effector applied to the accumulating Force of a stage, in EXACT arithmetic.  `kind` is E.kind for the run-time
 // interpreter and a compile-time constant for effector sequences (the switch then folds away).
-template <bool GREG>
+// SCHED: the launch carries input schedules; the effector's column is the row of `tick` (the tick being integrated)
+template <bool GREG, bool SCHED = false>
 __device__ __forceinline__ void apply_effector_exact(uint32_t kind, const EffDev &E, const StepParams &P, uint64_t b, int slot,
                                                      const Pose &sx, const ex::PoseInv &pi, const Motion &sv, const Inertia &I,
-                                                     const GravReg &greg, Motion &F)
+                                                     const GravReg &greg, Motion &F, uint64_t tick = 0)
 {
     using namespace ex;
+    // the column base at each use (unscheduled launches read E.col there, exactly as without schedules)
+    auto col = [&]() { return SCHED ? schedule_ptr(E.col, E.sched, tick) : E.col; };
     switch (kind) {
     case B200_EFF_GRAVITY_CONST: { // ball/sim.py:56-58: f + SpatialForce(linear=g*m)
         F.ang = Vec3{add(F.ang.x, 0.0), add(F.ang.y, 0.0), add(F.ang.z, 0.0)};
@@ -133,11 +136,11 @@ __device__ __forceinline__ void apply_effector_exact(uint32_t kind, const EffDev
     }
     case B200_EFF_DRAG_QUADRATIC: { // ball/sim.py:99-116; result torque is zero
         double w0 = 0.0, w1 = 0.0, w2 = 0.0;
-        if (E.col) { w0 = ldp(E.col, P.ld, 0, b); w1 = ldp(E.col, P.ld, 1, b); w2 = ldp(E.col, P.ld, 2, b); }
+        if (col()) { w0 = ldp(col(), P.ld, 0, b); w1 = ldp(col(), P.ld, 1, b); w2 = ldp(col(), P.ld, 2, b); }
         const Vec3 fl = {sub(w0, sv.lin.x), sub(w1, sv.lin.y), sub(w2, sv.lin.z)};
         const double speed = sqr(dot3(fl));
-        const double cd_rho = E.col_width == 5 ? ldp(E.col, P.ld, 3, b) : E.p[0];
-        const double area = E.col_width == 5 ? ldp(E.col, P.ld, 4, b) : E.p[1];
+        const double cd_rho = E.col_width == 5 ? ldp(col(), P.ld, 3, b) : E.p[0];
+        const double area = E.col_width == 5 ? ldp(col(), P.ld, 4, b) : E.p[1];
         const double drag = mul(0.5, mul(mul(cd_rho, mul(speed, speed)), area));
         const Vec3 dir = div3(fl, speed);
         F.ang = Vec3{0.0, 0.0, 0.0};
@@ -145,7 +148,7 @@ __device__ __forceinline__ void apply_effector_exact(uint32_t kind, const EffDev
         break;
     }
     case B200_EFF_THRUST_BODY: { // rocket/main.py:429-431
-        const double t = E.col ? ldp(E.col, P.ld, 0, b) : 0.0;
+        const double t = col() ? ldp(col(), P.ld, 0, b) : 0.0;
         const Vec3 d = qrot_with(sx.q, pi.qi, Vec3{E.p[0], E.p[1], E.p[2]});
         F.ang = Vec3{add(F.ang.x, 0.0), add(F.ang.y, 0.0), add(F.ang.z, 0.0)};
         F.lin = Vec3{add(F.lin.x, mul(d.x, t)), add(F.lin.y, mul(d.y, t)), add(F.lin.z, mul(d.z, t))};
@@ -153,9 +156,9 @@ __device__ __forceinline__ void apply_effector_exact(uint32_t kind, const EffDev
     }
     case B200_EFF_WRENCH_BODY: { // rocket/main.py:407-413, falcon9/sim.py:659-672
         Vec3 a = {0.0, 0.0, 0.0}, c = {0.0, 0.0, 0.0};
-        if (E.col) {
-            a = Vec3{ldp(E.col, P.ld, 0, b), ldp(E.col, P.ld, 1, b), ldp(E.col, P.ld, 2, b)};
-            c = Vec3{ldp(E.col, P.ld, 3, b), ldp(E.col, P.ld, 4, b), ldp(E.col, P.ld, 5, b)};
+        if (col()) {
+            a = Vec3{ldp(col(), P.ld, 0, b), ldp(col(), P.ld, 1, b), ldp(col(), P.ld, 2, b)};
+            c = Vec3{ldp(col(), P.ld, 3, b), ldp(col(), P.ld, 4, b), ldp(col(), P.ld, 5, b)};
         }
         const bool lin_first = (E.flags & B200_EFF_FLAG_WRENCH_LINEAR_FIRST) != 0;
         const Vec3 tw = qrot_with(sx.q, pi.qi, lin_first ? c : a);
@@ -180,19 +183,19 @@ __device__ __forceinline__ void apply_effector_exact(uint32_t kind, const EffDev
         break;
     }
     case B200_EFF_WRENCH_WORLD: { // cube-sat/main.py:516-527, drone/sim.py:99-103: force + SpatialForce(..)
-        if (E.col) {
-            F.ang = Vec3{add(F.ang.x, ldp(E.col, P.ld, 0, b)), add(F.ang.y, ldp(E.col, P.ld, 1, b)), add(F.ang.z, ldp(E.col, P.ld, 2, b))};
-            F.lin = Vec3{add(F.lin.x, ldp(E.col, P.ld, 3, b)), add(F.lin.y, ldp(E.col, P.ld, 4, b)), add(F.lin.z, ldp(E.col, P.ld, 5, b))};
+        if (col()) {
+            F.ang = Vec3{add(F.ang.x, ldp(col(), P.ld, 0, b)), add(F.ang.y, ldp(col(), P.ld, 1, b)), add(F.ang.z, ldp(col(), P.ld, 2, b))};
+            F.lin = Vec3{add(F.lin.x, ldp(col(), P.ld, 3, b)), add(F.lin.y, ldp(col(), P.ld, 4, b)), add(F.lin.z, ldp(col(), P.ld, 5, b))};
         }
         break;
     }
     case B200_EFF_TORQUE_BODY_FOLD: { // cube-sat/main.py:492-505: Force := fold_k (f + SpatialForce(torque = q @ tau_k))
-        if (E.col) {
+        if (col()) {
             Motion acc = {{0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}};
             const uint32_t K = E.col_width / 3u;
             for (uint32_t k = 0; k < K; ++k) {
-                const Vec3 t = qrot_with(sx.q, pi.qi, Vec3{ldp(E.col, P.ld, 3 * k + 0, b), ldp(E.col, P.ld, 3 * k + 1, b),
-                                                           ldp(E.col, P.ld, 3 * k + 2, b)});
+                const Vec3 t = qrot_with(sx.q, pi.qi, Vec3{ldp(col(), P.ld, 3 * k + 0, b), ldp(col(), P.ld, 3 * k + 1, b),
+                                                           ldp(col(), P.ld, 3 * k + 2, b)});
                 acc.ang = Vec3{add(acc.ang.x, t.x), add(acc.ang.y, t.y), add(acc.ang.z, t.z)};
                 acc.lin = Vec3{add(acc.lin.x, 0.0), add(acc.lin.y, 0.0), add(acc.lin.z, 0.0)};
             }
@@ -230,16 +233,16 @@ __device__ __forceinline__ void apply_effector_exact(uint32_t kind, const EffDev
 }
 
 // clear_forces | effectors (array order) on the stage state; six_dof.rs:148-150,195
-template <bool GREG>
+template <bool GREG, bool SCHED = false>
 __device__ __forceinline__ Motion effectors_exact(const StepParams &P, uint64_t b, int slot, const Pose &sx,
                                                   const ex::PoseInv &pi, const Motion &sv, const Inertia &I,
-                                                  const GravReg &greg)
+                                                  const GravReg &greg, uint64_t tick = 0)
 {
     Motion F = {{0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}};
     for (uint32_t e = 0; e < P.n_eff; ++e) {
         const EffDev &E = P.eff[e];
         if (E.mask && !E.mask[(b + P.ent0) % P.n_entities]) continue; // entity does not own the effector's components (query join)
-        apply_effector_exact<GREG>(E.kind, E, P, b, slot, sx, pi, sv, I, greg, F);
+        apply_effector_exact<GREG, SCHED>(E.kind, E, P, b, slot, sx, pi, sv, I, greg, F, tick);
     }
     return F;
 }
@@ -248,17 +251,17 @@ __device__ __forceinline__ Motion effectors_exact(const StepParams &P, uint64_t 
 // bits each (0 ends the list; SEQ = 0 is the empty list).  Same operations in the same order as the interpreter — the
 // order of accumulation is part of the arithmetic — without its loop, its switch, and the registers they pin.
 static constexpr uint32_t SEQ_INTERPRET = 0xffffffffu;
-template <uint32_t SEQ, bool GREG>
+template <uint32_t SEQ, bool GREG, bool SCHED = false>
 __device__ __forceinline__ Motion effectors_exact_seq(const StepParams &P, uint64_t b, int slot, const Pose &sx,
                                                       const ex::PoseInv &pi, const Motion &sv, const Inertia &I,
-                                                      const GravReg &greg)
+                                                      const GravReg &greg, uint64_t tick = 0)
 {
     Motion F = {{0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}};
-    if constexpr (((SEQ >> 0) & 15u) != 0) apply_effector_exact<GREG>((SEQ >> 0) & 15u, P.eff[0], P, b, slot, sx, pi, sv, I, greg, F);
-    if constexpr (((SEQ >> 4) & 15u) != 0) apply_effector_exact<GREG>((SEQ >> 4) & 15u, P.eff[1], P, b, slot, sx, pi, sv, I, greg, F);
-    if constexpr (((SEQ >> 8) & 15u) != 0) apply_effector_exact<GREG>((SEQ >> 8) & 15u, P.eff[2], P, b, slot, sx, pi, sv, I, greg, F);
-    if constexpr (((SEQ >> 12) & 15u) != 0) apply_effector_exact<GREG>((SEQ >> 12) & 15u, P.eff[3], P, b, slot, sx, pi, sv, I, greg, F);
-    if constexpr (((SEQ >> 16) & 15u) != 0) apply_effector_exact<GREG>((SEQ >> 16) & 15u, P.eff[4], P, b, slot, sx, pi, sv, I, greg, F);
+    if constexpr (((SEQ >> 0) & 15u) != 0) apply_effector_exact<GREG, SCHED>((SEQ >> 0) & 15u, P.eff[0], P, b, slot, sx, pi, sv, I, greg, F, tick);
+    if constexpr (((SEQ >> 4) & 15u) != 0) apply_effector_exact<GREG, SCHED>((SEQ >> 4) & 15u, P.eff[1], P, b, slot, sx, pi, sv, I, greg, F, tick);
+    if constexpr (((SEQ >> 8) & 15u) != 0) apply_effector_exact<GREG, SCHED>((SEQ >> 8) & 15u, P.eff[2], P, b, slot, sx, pi, sv, I, greg, F, tick);
+    if constexpr (((SEQ >> 12) & 15u) != 0) apply_effector_exact<GREG, SCHED>((SEQ >> 12) & 15u, P.eff[3], P, b, slot, sx, pi, sv, I, greg, F, tick);
+    if constexpr (((SEQ >> 16) & 15u) != 0) apply_effector_exact<GREG, SCHED>((SEQ >> 16) & 15u, P.eff[4], P, b, slot, sx, pi, sv, I, greg, F, tick);
     return F;
 }
 
@@ -267,9 +270,10 @@ __device__ __forceinline__ Motion effectors_exact_seq(const StepParams &P, uint6
 // divisions, more registers) or keep them a loop
 // SEQ: SEQ_INTERPRET = interpret P.eff[] at run time; anything else = the effector list as a compile-time sequence
 // (0 = no effectors: clear_forces only)
-template <int INTEG, bool GREG, bool UNR = false, uint32_t SEQ = SEQ_INTERPRET>
+// SCHED, tick: the launch carries input schedules, `tick` is the Tick column value of the tick integrated here
+template <int INTEG, bool GREG, bool UNR = false, uint32_t SEQ = SEQ_INTERPRET, bool SCHED = false>
 __device__ __forceinline__ void exact_tick(const StepParams &P, uint64_t b, Pose &x0, Motion &v0, Motion &a_out,
-                                           Motion &f_out, const Inertia &I, const GravReg &greg)
+                                           Motion &f_out, const Inertia &I, const GravReg &greg, uint64_t tick = 0)
 {
     using namespace ex;
     const InertiaRcp IR = inertia_rcp(I); // loop-invariant when a launch integrates several ticks
@@ -289,8 +293,8 @@ __device__ __forceinline__ void exact_tick(const StepParams &P, uint64_t b, Pose
             for (int j = 0; j < n_stages; ++j) {
                 const int s = (k == 0) ? 0 : (k == 1 ? 1 + j : 3);
                 const Motion sv = madd(v0, scale(dtf, sa));
-                if constexpr (SEQ == SEQ_INTERPRET) f_out = effectors_exact<GREG>(P, b, k, sx, pi, sv, I, greg);
-                else f_out = effectors_exact_seq<SEQ, GREG>(P, b, k, sx, pi, sv, I, greg);
+                if constexpr (SEQ == SEQ_INTERPRET) f_out = effectors_exact<GREG, SCHED>(P, b, k, sx, pi, sv, I, greg, tick);
+                else f_out = effectors_exact_seq<SEQ, GREG, SCHED>(P, b, k, sx, pi, sv, I, greg, tick);
                 sa = calc_accel_with(sx, pi, f_out, I, IR);
                 if (s == 0) { kv = sv; ka = sa; }
                 else if (s == 3) { kv = madd(kv, sv); ka = madd(ka, sa); }
@@ -304,8 +308,8 @@ __device__ __forceinline__ void exact_tick(const StepParams &P, uint64_t b, Pose
     } else {
         // semi_implicit.rs:42-62
         const PoseInv pi = pose_inverses(x0.q);
-        if constexpr (SEQ == SEQ_INTERPRET) f_out = effectors_exact<GREG>(P, b, 0, x0, pi, v0, I, greg);
-        else f_out = effectors_exact_seq<SEQ, GREG>(P, b, 0, x0, pi, v0, I, greg);
+        if constexpr (SEQ == SEQ_INTERPRET) f_out = effectors_exact<GREG, SCHED>(P, b, 0, x0, pi, v0, I, greg, tick);
+        else f_out = effectors_exact_seq<SEQ, GREG, SCHED>(P, b, 0, x0, pi, v0, I, greg, tick);
         a_out = calc_accel_with(x0, pi, f_out, I, IR);
         v0 = madd(v0, scale(P.dt_final, a_out));
         x0 = tadd(x0, scale(P.dt_final, v0));
@@ -369,9 +373,10 @@ struct Folded {
     bool aforce;        // GRAVITY_EGM08: add the stage-force planes egm08_force_kernel filled
 };
 
-template <bool GREG>
+// SCHED: the launch carries input schedules; effector columns are read at the row of `tick`
+template <bool GREG, bool SCHED = false>
 __device__ __forceinline__ Folded fold_effectors(const StepParams &P, uint64_t b, const Inertia &I, const Vec3 &invI,
-                                                 const GravReg &greg)
+                                                 const GravReg &greg, uint64_t tick = 0)
 {
     Folded f;
     f.fw = f.fb = f.u = f.wind = f.om = Vec3{0.0, 0.0, 0.0};
@@ -382,27 +387,28 @@ __device__ __forceinline__ Folded fold_effectors(const StepParams &P, uint64_t b
     for (uint32_t e = 0; e < P.n_eff; ++e) {
         const EffDev &E = P.eff[e];
         if (E.mask && !E.mask[(b + P.ent0) % P.n_entities]) continue; // query join: not a member
+        auto col = [&]() { return SCHED ? schedule_ptr(E.col, E.sched, tick) : E.col; }; // read at each use, like E.col
         switch (E.kind) {
         case B200_EFF_GRAVITY_CONST:
             f.fw.x = fma(E.p[0], I.m, f.fw.x); f.fw.y = fma(E.p[1], I.m, f.fw.y); f.fw.z = fma(E.p[2], I.m, f.fw.z);
             break;
         case B200_EFF_DRAG_QUADRATIC:
             f.drag = true;
-            f.kd = E.col_width == 5 ? 0.5 * ldp(E.col, P.ld, 3, b) * ldp(E.col, P.ld, 4, b) : 0.5 * E.p[0] * E.p[1];
-            if (E.col) f.wind = Vec3{ldp(E.col, P.ld, 0, b), ldp(E.col, P.ld, 1, b), ldp(E.col, P.ld, 2, b)};
+            f.kd = E.col_width == 5 ? 0.5 * ldp(col(), P.ld, 3, b) * ldp(col(), P.ld, 4, b) : 0.5 * E.p[0] * E.p[1];
+            if (col()) f.wind = Vec3{ldp(col(), P.ld, 0, b), ldp(col(), P.ld, 1, b), ldp(col(), P.ld, 2, b)};
             tb = Vec3{0.0, 0.0, 0.0}; // the reference's apply_drag returns SpatialForce(linear=...): torque reset
             break;
         case B200_EFF_THRUST_BODY: {
-            const double t = E.col ? ldp(E.col, P.ld, 0, b) : 0.0;
+            const double t = col() ? ldp(col(), P.ld, 0, b) : 0.0;
             f.fb.x = fma(E.p[0], t, f.fb.x); f.fb.y = fma(E.p[1], t, f.fb.y); f.fb.z = fma(E.p[2], t, f.fb.z);
             break;
         }
         case B200_EFF_WRENCH_BODY:
-            if (E.col) {
+            if (col()) {
                 const int to = (E.flags & B200_EFF_FLAG_WRENCH_LINEAR_FIRST) ? 3 : 0;
                 const int fo = 3 - to;
-                tb.x += ldp(E.col, P.ld, to + 0, b); tb.y += ldp(E.col, P.ld, to + 1, b); tb.z += ldp(E.col, P.ld, to + 2, b);
-                f.fb.x += ldp(E.col, P.ld, fo + 0, b); f.fb.y += ldp(E.col, P.ld, fo + 1, b); f.fb.z += ldp(E.col, P.ld, fo + 2, b);
+                tb.x += ldp(col(), P.ld, to + 0, b); tb.y += ldp(col(), P.ld, to + 1, b); tb.z += ldp(col(), P.ld, to + 2, b);
+                f.fb.x += ldp(col(), P.ld, fo + 0, b); f.fb.y += ldp(col(), P.ld, fo + 1, b); f.fb.z += ldp(col(), P.ld, fo + 2, b);
             }
             break;
         case B200_EFF_GRAVITY_FRAME:
@@ -411,20 +417,20 @@ __device__ __forceinline__ Folded fold_effectors(const StepParams &P, uint64_t b
             f.om = Vec3{E.p[1], E.p[2], E.p[3]};
             break;
         case B200_EFF_WRENCH_WORLD:
-            if (E.col) {
-                f.tw.x += ldp(E.col, P.ld, 0, b); f.tw.y += ldp(E.col, P.ld, 1, b); f.tw.z += ldp(E.col, P.ld, 2, b);
-                f.fw.x += ldp(E.col, P.ld, 3, b); f.fw.y += ldp(E.col, P.ld, 4, b); f.fw.z += ldp(E.col, P.ld, 5, b);
+            if (col()) {
+                f.tw.x += ldp(col(), P.ld, 0, b); f.tw.y += ldp(col(), P.ld, 1, b); f.tw.z += ldp(col(), P.ld, 2, b);
+                f.fw.x += ldp(col(), P.ld, 3, b); f.fw.y += ldp(col(), P.ld, 4, b); f.fw.z += ldp(col(), P.ld, 5, b);
                 f.wtorque = true;
             }
             break;
         case B200_EFF_TORQUE_BODY_FOLD: // Force := fold: everything accumulated before it is overwritten
-            if (E.col) {
+            if (col()) {
                 tb = Vec3{0.0, 0.0, 0.0};
                 f.fw = f.fb = f.tw = Vec3{0.0, 0.0, 0.0};
                 f.drag = f.frame = f.wtorque = f.j2 = f.aforce = false;
                 const uint32_t K = E.col_width / 3u;
                 for (uint32_t k = 0; k < K; ++k) {
-                    tb.x += ldp(E.col, P.ld, 3 * k + 0, b); tb.y += ldp(E.col, P.ld, 3 * k + 1, b); tb.z += ldp(E.col, P.ld, 3 * k + 2, b);
+                    tb.x += ldp(col(), P.ld, 3 * k + 0, b); tb.y += ldp(col(), P.ld, 3 * k + 1, b); tb.z += ldp(col(), P.ld, 3 * k + 2, b);
                 }
             }
             break;
@@ -445,6 +451,38 @@ __device__ __forceinline__ Folded fold_effectors(const StepParams &P, uint64_t b
     }
     f.u = Vec3{tb.x * invI.x, tb.y * invI.y, tb.z * invI.z};
     return f;
+}
+
+// the per-body inputs of signature SIG at the schedule rows of `tick` (fused launches with input schedules: every tick
+// after the first reloads them; the first tick's inputs arrive with the state loads)
+template <uint32_t SIG>
+__device__ __forceinline__ EffIn load_spec_inputs(const StepParams &P, uint64_t b, uint64_t tick)
+{
+    EffIn in;
+    in.thrust = 0.0; in.cd_rho = in.area = 0.0;
+    in.wr_t = in.wr_f = in.wind = in.wheels = in.ww_t = in.ww_f = Vec3{0.0, 0.0, 0.0};
+    if (SIG & SIG_THRUST) in.thrust = ldp(schedule_ptr(P.spec.thrust, P.spec.s_thrust, tick), P.ld, 0, b);
+    if (SIG & SIG_WRENCH) {
+        const double *t = schedule_ptr(P.spec.wr_t, P.spec.s_wrench, tick), *f = schedule_ptr(P.spec.wr_f, P.spec.s_wrench, tick);
+        in.wr_t = Vec3{ldp(t, P.ld, 0, b), ldp(t, P.ld, 1, b), ldp(t, P.ld, 2, b)};
+        in.wr_f = Vec3{ldp(f, P.ld, 0, b), ldp(f, P.ld, 1, b), ldp(f, P.ld, 2, b)};
+    }
+    if (SIG & SIG_WHEELS) { // summed in the order the kernel's initial load sums them
+        const double *w = schedule_ptr(P.spec.wheels, P.spec.s_wheels, tick);
+        in.wheels = Vec3{ldp(w, P.ld, 0, b) + ldp(w, P.ld, 3, b) + ldp(w, P.ld, 6, b), ldp(w, P.ld, 1, b) + ldp(w, P.ld, 4, b) + ldp(w, P.ld, 7, b),
+                         ldp(w, P.ld, 2, b) + ldp(w, P.ld, 5, b) + ldp(w, P.ld, 8, b)};
+    }
+    if (SIG & SIG_WWORLD) {
+        const double *w = schedule_ptr(P.spec.wworld, P.spec.s_wworld, tick);
+        in.ww_t = Vec3{ldp(w, P.ld, 0, b), ldp(w, P.ld, 1, b), ldp(w, P.ld, 2, b)};
+        in.ww_f = Vec3{ldp(w, P.ld, 3, b), ldp(w, P.ld, 4, b), ldp(w, P.ld, 5, b)};
+    }
+    if (SIG & SIG_DRAG) {
+        const double *d = schedule_ptr(P.spec.drag, P.spec.s_drag, tick);
+        in.wind = Vec3{ldp(d, P.ld, 0, b), ldp(d, P.ld, 1, b), ldp(d, P.ld, 2, b)};
+        if (SIG & SIG_DRAG_PB) { in.cd_rho = ldp(d, P.ld, 3, b); in.area = ldp(d, P.ld, 4, b); }
+    }
+    return in;
 }
 
 // the same fold for a compile-time signature: constants from StepParams::spec (constant bank), per-body inputs
@@ -561,7 +599,9 @@ __device__ __forceinline__ Motion force_out_fast(const Vec3 &a_lin, const Vec3 &
 // n_ticks ticks of one body, state in registers (shared by the direct and the TMA-pipelined kernel)
 // (n_ticks, tick0, want_f) are P.n_ticks, P.tick0, P.write_fa for the kernels that integrate a launch's ticks
 // in one call; small_world_kernel calls it once per tick with that tick's gravity in `greg`
-template <int INTEG, bool TRAJ, bool GREG = false, uint32_t SIG = SIG_GENERIC>
+// SCHED: the launch carries input schedules (P.sched): tick t of the launch (Tick value P.tick_abs + t) folds the
+// effector inputs of its own schedule rows; `in` holds the first tick's
+template <int INTEG, bool TRAJ, bool GREG = false, uint32_t SIG = SIG_GENERIC, bool SCHED = false>
 __device__ __forceinline__ void fast_ticks(const StepParams &P, uint64_t b, Pose &x0, Motion &v0, const Inertia &I,
                                            Motion &a_last, Motion &f_last, uint32_t n_ticks, uint64_t tick0, bool want_f,
                                            const GravReg &greg, const EffIn &in = EffIn{}, bool store_traj = true)
@@ -571,7 +611,7 @@ __device__ __forceinline__ void fast_ticks(const StepParams &P, uint64_t b, Pose
     const Vec3 invI = NEED_INVI ? Vec3{fa::rcp_nr(I.diag.x), fa::rcp_nr(I.diag.y), fa::rcp_nr(I.diag.z)} : Vec3{0.0, 0.0, 0.0};
     const double inv_m = fa::rcp_nr(I.m);
     Folded f;
-    if constexpr (GEN) f = fold_effectors<GREG>(P, b, I, invI, greg);
+    if constexpr (GEN) f = fold_effectors<GREG, SCHED>(P, b, I, invI, greg, P.tick_abs);
     else f = fold_spec<SIG, GREG>(P, b, in, I, invI, greg);
 
     a_last = Motion{{0.0, 0.0, 0.0}, {0.0, 0.0, 0.0}};
@@ -579,9 +619,10 @@ __device__ __forceinline__ void fast_ticks(const StepParams &P, uint64_t b, Pose
     const double dt = P.dt_stage;
     // generic: data-dependent (most bodies of a heterogeneous world carry no body-frame wrench; NaNs compare
     // unequal to zero and take the full path); specialised: a property of the signature
-    const bool has_u = GEN ? ((f.u.x != 0.0) | (f.u.y != 0.0) | (f.u.z != 0.0)) : (SIG & (SIG_WRENCH | SIG_WHEELS)) != 0;
-    const bool has_fb = GEN ? ((f.fb.x != 0.0) | (f.fb.y != 0.0) | (f.fb.z != 0.0)) : (SIG & (SIG_THRUST | SIG_WRENCH)) != 0;
-    const bool has_tw = GEN ? f.wtorque : (SIG & SIG_WWORLD) != 0; // world-frame torque: a_ang = R (invI .* (R^-1 tau_w)) per stage attitude
+    // (a scheduled interpreter launch re-derives them with every tick's fold)
+    bool has_u = GEN ? ((f.u.x != 0.0) | (f.u.y != 0.0) | (f.u.z != 0.0)) : (SIG & (SIG_WRENCH | SIG_WHEELS)) != 0;
+    bool has_fb = GEN ? ((f.fb.x != 0.0) | (f.fb.y != 0.0) | (f.fb.z != 0.0)) : (SIG & (SIG_THRUST | SIG_WRENCH)) != 0;
+    bool has_tw = GEN ? f.wtorque : (SIG & SIG_WWORLD) != 0; // world-frame torque: a_ang = R (invI .* (R^-1 tau_w)) per stage attitude
     auto ang_world = [&](const Quat &q) { // angular acceleration the world-frame torque produces at attitude q
         const Vec3 tbody = fa::rot(Quat{-q.i, -q.j, -q.k, q.w}, f.tw);
         return fa::rot(q, Vec3{tbody.x * invI.x, tbody.y * invI.y, tbody.z * invI.z});
@@ -594,6 +635,18 @@ __device__ __forceinline__ void fast_ticks(const StepParams &P, uint64_t b, Pose
     if (TRAJ && P.traj_every) { traj_phase = (uint32_t)(tick0 % P.traj_every); traj_slot = tick0 / P.traj_every; }
 
     for (uint32_t t = 0; t < n_ticks; ++t) {
+        if constexpr (SCHED) {
+            if (t > 0) {
+                if constexpr (GEN) {
+                    f = fold_effectors<GREG, true>(P, b, I, invI, greg, P.tick_abs + t);
+                    has_u = (f.u.x != 0.0) | (f.u.y != 0.0) | (f.u.z != 0.0);
+                    has_fb = (f.fb.x != 0.0) | (f.fb.y != 0.0) | (f.fb.z != 0.0);
+                    has_tw = f.wtorque;
+                } else {
+                    f = fold_spec<SIG, GREG>(P, b, load_spec_inputs<SIG>(P, b, P.tick_abs + t), I, invI, greg);
+                }
+            }
+        }
         if (INTEG == B200_INTEGRATOR_RK4) {
             const Vec3 w0 = v0.ang, u0 = v0.lin;
             // the three distinct stage poses depend on (x0, v0) only (rk4.rs:85-111)

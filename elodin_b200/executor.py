@@ -158,6 +158,24 @@ class B200Exec:
         for name, a in columns.items():
             self.upload(name, a)
 
+    # ---- input schedules ----------------------------------------------------------
+    def set_schedule(self, cid, rows, first_tick: int = 0) -> None:
+        """Drive effector input column `cid` from per-tick rows held on the device: `rows` is
+        [T, n_worlds, n_entities, width]; the tick whose Tick value is k reads row clamp(k - first_tick, 0, T - 1).
+        Replaces an earlier schedule of the column.  See b200_sixdof_set_schedule."""
+        cid = _cid(cid)
+        a = np.ascontiguousarray(rows, dtype=np.float64)
+        if a.ndim != 4 or a.shape[0] < 1:
+            raise _lib.B200ValueError(_lib.ERR_VALUE_SIZE_MISMATCH,
+                                      f"schedule rows must be [T >= 1, n_worlds, n_entities, width], got shape {a.shape}")
+        if first_tick < 0:
+            raise ValueError(f"first_tick must be >= 0, got {first_tick}")
+        _lib.check(self._L.b200_sixdof_set_schedule(self._h, cid, a.ctypes.data, a.nbytes, a.shape[0], int(first_tick)))
+
+    def clear_schedule(self, cid) -> None:
+        """Unbind the schedule of `cid`: the column keeps the row its last tick used, later ticks read the column."""
+        _lib.check(self._L.b200_sixdof_clear_schedule(self._h, _cid(cid)))
+
     # ---- stepping ---------------------------------------------------------------
     def step(self, n_ticks: int = 1, sync: bool = False) -> None:
         _lib.check(self._L.b200_sixdof_step(self._h, int(n_ticks)))
@@ -170,7 +188,8 @@ class B200Exec:
     def invoke_batch(self, in_cols: Sequence[np.ndarray], n_ticks: int = 1,
                      out_cols: Optional[Sequence[np.ndarray]] = None):
         """CraneliftExec::invoke_batch (cranelift_exec.rs:129-195): `in_cols[i]` is the
-        host buffer of `input_ids[i]`; returns the buffers of `output_ids`."""
+        host buffer of `input_ids[i]` (None: not dirty; always None for a scheduled column);
+        returns the buffers of `output_ids`."""
         if len(in_cols) != len(self.input_ids):
             raise _lib.B200ValueError(_lib.ERR_VALUE_SIZE_MISMATCH, "wrong number of input columns")
         ins = []

@@ -290,13 +290,63 @@ class HostSystem(System):
     """A per-tick host callback over the numpy columns (non-effector systems such as
     the rocket's thrust curve, examples/rocket/main.py:416-426).  It runs on the host
     between GPU ticks, like copy_db_to_world feeding external controls
-    (impeller2_server.rs:607), and forces one tick per launch."""
+    (impeller2_server.rs:607), and forces one tick per launch.  An input known ahead of
+    time and indexed by tick (a thrust curve) runs faster as an input_schedule()."""
 
     fn: Callable[["StepContext"], None]
 
 
 def host_system(fn) -> HostSystem:
     return HostSystem(fn)
+
+
+@dataclasses.dataclass(eq=False)
+class InputSchedule(System):
+    """Per-tick rows of an effector input column, held on the device (B200Exec.set_schedule): a thrust curve, a
+    recorded wind or a per-world open-loop profile without a host callback, so the run keeps the device-resident
+    route and fused ticks."""
+
+    component: str
+    rows: np.ndarray
+    first_tick: int = 0
+
+
+def input_schedule(component, rows, first_tick: int = 0) -> InputSchedule:
+    """`el.input_schedule("thrust", rows, first_tick=0) | el.six_dof(...)`: the tick whose Tick value is k sees
+    row clamp(k - first_tick, 0, T - 1) in the effector input column `component` — the same values a host_system
+    writing `rows[tick]` before every tick would leave there.  `rows` is [T, n_owner_entities(, width)] (one curve
+    for every world) or [T, n_worlds, n_owner_entities, width]; owner entities are the ones that carry the component,
+    in spawn order."""
+    if isinstance(component, Component):
+        name = component.name
+    elif isinstance(component, str):
+        name = component
+    else:
+        name = Component.of(component).name
+    if int(first_tick) < 0:
+        raise ValueError(f"input_schedule({name!r}): first_tick must be >= 0, got {first_tick}")
+    return InputSchedule(name, np.asarray(rows, dtype=np.float64), int(first_tick))
+
+
+def schedule_row(tick, first_tick: int, n_rows: int):
+    """Row of an input schedule that the tick whose Tick value is `tick` reads (scalar or array of ticks); the rule
+    of b200_sixdof_set_schedule."""
+    return np.clip(np.asarray(tick, dtype=np.int64) - int(first_tick), 0, int(n_rows) - 1)
+
+
+def _schedule_rows(name: str, rows: np.ndarray, n_worlds: int, n_owner: int, width: int) -> np.ndarray:
+    """[T, n_worlds, n_owner, width] from the shapes input_schedule accepts (broadcast over worlds on the host)."""
+    a = np.asarray(rows, dtype=np.float64)
+    if a.ndim == 2 and width == 1:
+        a = a[:, :, None]
+    if a.ndim == 3 and a.shape[1:] == (n_owner, width):
+        a = np.broadcast_to(a[:, None], (a.shape[0], n_worlds, n_owner, width))
+    elif not (a.ndim == 4 and a.shape[1:] == (n_worlds, n_owner, width)):
+        want = f"[T, {n_owner}, {width}] or [T, {n_worlds}, {n_owner}, {width}]" + (f" or [T, {n_owner}]" if width == 1 else "")
+        raise ValueError(f"input_schedule({name!r}): rows of shape {a.shape}, expected {want}")
+    if a.shape[0] < 1:
+        raise ValueError(f"input_schedule({name!r}): the schedule needs at least one row")
+    return np.ascontiguousarray(a)
 
 
 class StepContext:
@@ -307,13 +357,21 @@ class StepContext:
     def tick(self) -> int:
         return self._exec.tick
 
+    def _unscheduled(self, name: str) -> int:
+        cid = component_id(name)
+        if cid in self._exec._schedules:
+            raise ValueError(f"column '{name}' is driven by an input_schedule: a host system cannot read or write it")
+        return cid
+
     def column(self, name: str) -> np.ndarray:
         """[n_worlds, n_entities_with_component, width] numpy view of a host column."""
-        return self._exec.world.columns[component_id(name)].buffer
+        cid = self._unscheduled(name)
+        return self._exec.world.columns[cid].buffer
 
     def write_component(self, pair_name: str, value) -> None:
         ent, comp = pair_name.rsplit(".", 1)
-        col = self._exec.world.columns[component_id(comp)]
+        cid = self._unscheduled(comp)
+        col = self._exec.world.columns[cid]
         row = col.row_of(self._exec.world.entity_by_name(ent))
         col.buffer[:, row, :] = np.asarray(value, dtype=col.buffer.dtype).reshape(-1)
         self._exec.dirty.add(col.component.id)
@@ -520,10 +578,13 @@ class Exec:
         pre = systems[: systems.index(self.six)]
         post = systems[systems.index(self.six) + 1:]
         for s in pre + post:
-            if not isinstance(s, HostSystem):
+            if not isinstance(s, (HostSystem, InputSchedule)):
                 raise _lib.B200Error(_lib.ERR_UNSUPPORTED,
                                      f"{s!r}: only host_system() callbacks may surround six_dof() (no tracing compiler)")
-        self.pre_systems, self.post_systems = pre, post
+            if isinstance(s, InputSchedule) and s in post:
+                raise _lib.B200Error(_lib.ERR_UNSUPPORTED, f"input_schedule({s.component!r}) must come before six_dof()")
+        schedules = [s for s in pre if isinstance(s, InputSchedule)]
+        self.pre_systems, self.post_systems = [s for s in pre if isinstance(s, HostSystem)], post
         # The reference's build yields an independent exec: this one owns private copies of the world's columns
         # (a later World.build() re-finalises the World's own buffers) and of the effector objects (the query-join
         # masks below are per build — the caller's effectors are never mutated).
@@ -538,6 +599,20 @@ class Exec:
         self.ticks_per_telemetry = ticks_per_telemetry(simulation_rate, telemetry_rate)
         self.max_ticks = max_ticks
         world.finalize(self.n_worlds)
+        # input schedules: cid -> (rows [T, n_worlds, n_owner, width], first_tick); the host keeps the rows for history
+        self._schedules: Dict[int, tuple] = {}
+        effector_cols = {component_id(e.column_name()) for e in self._effectors if e.column_name()}
+        for s in schedules:
+            cid = component_id(s.component)
+            if cid in self._schedules:
+                raise ValueError(f"two input_schedule()s drive column '{s.component}'")
+            if cid not in effector_cols:
+                raise ValueError(f"input_schedule({s.component!r}): not an input column of a six_dof() effector")
+            if (world_params or {}).keys() & {s.component}:
+                raise ValueError(f"world_params sets column '{s.component}', which an input_schedule drives")
+            col = world.columns[cid]
+            self._schedules[cid] = (_schedule_rows(s.component, s.rows, self.n_worlds, len(col.entity_ids), col.width),
+                                    s.first_tick)
         for name, arr in (world_params or {}).items():
             col = world.columns[component_id(name)]
             col.buffer[...] = np.asarray(arr, dtype=col.dtype).reshape(col.buffer.shape)
@@ -583,6 +658,12 @@ class Exec:
                                 self.six.integrator.value, math, device, max_fused_ticks=32, world=world,
                                 trajectory_every=self.ticks_per_telemetry if self._ring_cap else 0,
                                 trajectory_capacity=self._ring_cap, trajectory_full=bool(self._ring_cap))
+        for cid, (rows, first) in self._schedules.items():
+            if cid in self._partial:  # body-row-expanded like the column the device holds
+                full = np.zeros(rows.shape[:2] + (len(bodies), rows.shape[3]))
+                full[:, :, self._partial[cid][0], :] = rows
+                rows = full
+            self.backend.set_schedule(cid, rows, first)
         self.tick = 0
         self.build_ms = 0.0
         self._prof = {"execute_buffers": [], "add_to_history": [], "h2d_upload": [], "kernel_invoke": [], "d2h_download": []}
@@ -593,6 +674,11 @@ class Exec:
         self._record()
 
     # -- data plumbing -------------------------------------------------------------
+    def _scheduled_value(self, cid: int, tick):
+        """Host value of a scheduled column after the tick whose Tick value is `tick` (array: one per tick)."""
+        rows, first = self._schedules[cid]
+        return rows[schedule_row(tick, first, rows.shape[0])]
+
     def _record(self) -> None:
         for cid, col in self.world.columns.items():
             self._history[cid].append(col.buffer.copy())
@@ -613,6 +699,8 @@ class Exec:
                 self._ins.append(self._tick_in)
             elif cid == component_id("simulation_time_step"):
                 self._ins.append(self._dt_in)
+            elif cid in self._schedules:
+                self._ins.append(None)  # the device-resident schedule drives it
             elif cid in self._partial:
                 self._ins.append(self._partial[cid][1])  # body-row-expanded copy, refreshed before every invoke
             else:
@@ -622,12 +710,14 @@ class Exec:
         for cid in be.output_ids:
             if cid in (component_id("tick"), component_id("simulation_time_step")):
                 self._outs.append(np.zeros(1, dtype=np.uint64 if cid == component_id("tick") else np.float64))
+            elif cid in self._schedules:
+                self._outs.append(None)  # known on the host: the row of the last tick
             elif cid in self._partial:
                 self._outs.append(np.empty_like(self._partial[cid][1]))
             else:
                 self._outs.append(np.empty_like(self.world.columns[cid].buffer))
-        self._in_ptrs = [a.ctypes.data for a in self._ins]
-        self._out_ptrs = [a.ctypes.data for a in self._outs]
+        self._in_ptrs = [None if a is None else a.ctypes.data for a in self._ins]
+        self._out_ptrs = [None if a is None else a.ctypes.data for a in self._outs]
 
     def _invoke(self, n: int) -> None:
         """WorldExec::run -> invoke_batch (cranelift_exec.rs:284-303,129-195)."""
@@ -637,16 +727,19 @@ class Exec:
         self._tick_in[0] = self.tick
         self._dt_in[0] = self.sim_time_step
         for cid, (rows, expanded) in self._partial.items():
-            expanded[:, rows, :] = self.world.columns[cid].buffer
+            if cid not in self._schedules:
+                expanded[:, rows, :] = self.world.columns[cid].buffer
         be.invoke_batch_ptrs(self._in_ptrs, self._out_ptrs, n)
         for cid, buf in zip(be.output_ids, self._outs):
             if cid == component_id("tick"):
                 self.tick = int(buf[0])  # world.advance_tick() x n
-            elif cid != component_id("simulation_time_step") and cid not in self._partial:
+            elif cid != component_id("simulation_time_step") and cid not in self._partial and buf is not None:
                 col = self.world.columns[cid]
                 if col.buffer.nbytes != buf.nbytes:
                     raise _lib.B200ValueError(_lib.ERR_VALUE_SIZE_MISMATCH, "value size mismatch")
                 np.copyto(col.buffer, buf)
+        for cid in self._schedules:
+            np.copyto(self.world.columns[cid].buffer, self._scheduled_value(cid, self.tick - 1))
 
     def _run_resident(self, cycles: int) -> None:
         """`cycles` whole telemetry cycles without leaving the device: upload the host columns once, step,
@@ -660,6 +753,8 @@ class Exec:
                 be.upload(cid, np.array([self.tick], dtype=np.uint64))
             elif cid == dt_id:
                 be.upload(cid, np.array([self.sim_time_step]))
+            elif cid in self._schedules:
+                continue  # the device-resident schedule drives it
             elif cid in self._partial:
                 rows, expanded = self._partial[cid]
                 expanded[:, rows, :] = self.world.columns[cid].buffer
@@ -681,8 +776,13 @@ class Exec:
             t_hist = time.perf_counter()
             for cid, lo, hi in body_cols:                            # one contiguous block per column, rows are views
                 self._history[cid].extend(np.ascontiguousarray(traj[:, :, :, lo:hi]))
+            last_ticks = self.tick + (np.arange(c) + 1) * tpt - 1         # Tick value of each cycle's last tick
             for cid, col in self.world.columns.items():
-                if cid not in sampled:                               # not written by six_dof(): pass-through
+                if cid in self._schedules:                           # the row each cycle's last tick used
+                    vals = self._scheduled_value(cid, last_ticks)
+                    self._history[cid].extend(vals)
+                    np.copyto(col.buffer, vals[-1])
+                elif cid not in sampled:                             # not written by six_dof(): pass-through
                     self._history[cid].extend([col.buffer.copy()] * c)
             self._globals_hist.extend((self.tick + (k + 1) * tpt, self.sim_time_step) for k in range(c))
             self.tick += c * tpt

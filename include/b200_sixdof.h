@@ -240,6 +240,25 @@ uint64_t b200_sixdof_column_bytes(const b200_sixdof *h, uint64_t component_id);
 int b200_sixdof_upload(b200_sixdof *h, uint64_t component_id, const void *src, uint64_t bytes);
 int b200_sixdof_download(b200_sixdof *h, uint64_t component_id, void *dst, uint64_t bytes);
 
+/* Input schedules: drive an effector input column from a table of per-tick rows held on the device, so that a
+ * thrust curve, a recorded input or a per-world open-loop profile runs in fused, device-resident launches.
+ *   rows        n_rows rows, each in the column's host layout [n_worlds][n_entities][width] f64, so
+ *               bytes == n_rows * b200_sixdof_column_bytes (else B200_ERR_VALUE_SIZE_MISMATCH).  Copied at this call.
+ *   row rule    the tick whose Tick column value is k reads row clamp(k - first_tick, 0, n_rows - 1): the first row
+ *               before the table starts, the last one after it ends.  k is the Tick value (invoke_batch: the `tick`
+ *               input it is handed), not the trajectory tick count a trajectory reset restarts.
+ *   readback    after ticks, the column (download, invoke_batch output) reads back as the row its last tick used.
+ *   inputs      invoke_batch refuses a non-NULL input for a scheduled column, and upload refuses the column
+ *               (B200_ERR_INVALID_ARGUMENT): the schedule owns it.
+ * Only effector input columns take a schedule (state columns and the globals: B200_ERR_INVALID_ARGUMENT).  Graph
+ * worlds (an edge_fold gravity effector) are B200_ERR_UNSUPPORTED, as is b200_sixdof_step_row_sharded while a
+ * schedule is bound.  Setting a scheduled column again replaces its schedule.  Clearing leaves the column holding its
+ * last-used row; later ticks read the column again.  The table takes n_rows * width * plane stride * 8 bytes of
+ * device memory (B200_ERR_OUT_OF_MEMORY if that fails). */
+int b200_sixdof_set_schedule(b200_sixdof *h, uint64_t component_id, const void *rows, uint64_t bytes, uint64_t n_rows,
+                             uint64_t first_tick);
+int b200_sixdof_clear_schedule(b200_sixdof *h, uint64_t component_id);
+
 /* Advance the device-resident world n_ticks (asynchronous on the handle's
  * stream).  tick += n_ticks. */
 int b200_sixdof_step(b200_sixdof *h, uint64_t n_ticks);
